@@ -2,6 +2,7 @@
 """Benchmark of the per-cell chrM pileup hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          our arm (CUDA, C-ABI)
+    python bench.py ... --dump-outputs DIR                       also write the last timed step's result to DIR/*.npy
     python bench.py --impl reference [...]                       the reference's own Python (baseline/_ref), C port beside it
     torchrun ... bench.py --gpus N --scaling strong              ONE configs[2]-shaped input split by barcode over N GPUs
 
@@ -45,7 +46,9 @@ def parse():
     ap.add_argument("--params", default="run", choices=["run", "tenx", "stress"],
                     help="filter set: run defaults (the bench line), tenx (configs[3]) or stress (configs[4]); "
                          "anything but `run` is a side measurement, not the bench line")
-    ap.add_argument("--e2e-steps", type=int, default=8)
+    ap.add_argument("--e2e-steps", type=int, default=None, help="timed steps of each e2e measurement (default: --steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed to DIR/<name>.npy (see dump_outputs)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--verify", action="store_true", help="check per-cell QC rows against the oracle at full size")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
@@ -55,7 +58,12 @@ def parse():
     ap.add_argument("--strong-records", type=int, default=200_000_000)
     ap.add_argument("--strong-parts", type=int, default=8, help="the strong-scaling input is the union of this many "
                     "barcode-disjoint parts (seeded per part, so it is the same input whatever the number of ranks)")
-    return ap.parse_args()
+    a = ap.parse_args()
+    if a.e2e_steps is None:
+        a.e2e_steps = a.steps
+    if a.steps < 1 or a.e2e_steps < 1:
+        ap.error("--steps and --e2e-steps must be at least 1")
+    return a
 
 
 def config_dict(a, n_gpus):
@@ -270,6 +278,39 @@ class ClockSampler:
                 "samples": len(self.samples), "power_w_max": max(self.power) if self.power else None}
 
 
+# --------------------------------------------------------------------------- outputs
+DUMP_CELLS = 40          # planes of this many cells: 40 x 11 x 16569 float64 = 58 MB, the rest of a dump is below 1 MB
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(res, out_dir):
+    """Write the PileupResult of a step (what a caller of the path receives) as .npy files of fixed shapes, so that two
+    builds can be compared output for output on the same seeded input:
+      planes.npy          float64 [DUMP_CELLS, 11, P]  exact planes (PLANE_NAMES order; entries saturated in the uint16
+                                                       planes carry their value from the overflow list, as counts() / tn5()
+                                                       / coverage() give them) of a fixed, seeded sample of cells;
+                                                       planes_cells.npy (float64) lists the sampled rows
+      cell_qc_<f>.npy     float64 [n_cells]            every field of the per-cell QC rows
+      base_totals.npy     float64 [P, 4]
+      stats.npy           float64 [8]                  STATS_FIELDS order
+    Every value is an integer below 2**53, so the float64 copies are exact."""
+    from mgatk2_b200._lib import N_PLANES
+    from mgatk2_b200.engine import STATS_FIELDS
+    n_cells = len(res.planes)
+    rows = np.sort(np.random.default_rng(BASE_SEED).choice(n_cells, min(n_cells, DUMP_CELLS), replace=False))
+    arrays = {"planes": np.stack([res.plane(k)[rows] for k in range(N_PLANES)], axis=1).astype(np.float64),
+              "planes_cells": rows.astype(np.float64),
+              **{f"cell_qc_{f}": res.cell_qc[f].astype(np.float64) for f in res.cell_qc.dtype.names},
+              "base_totals": res.base_totals.astype(np.float64),
+              "stats": np.array([res.stats[k] for k in STATS_FIELDS], np.float64)}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_LIMIT})")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), v)
+
+
 # --------------------------------------------------------------------------- our arm
 def run_b200(a):
     import torch
@@ -346,6 +387,7 @@ def run_b200(a):
     e1.record()
     barrier()
     ms_total = e0.elapsed_time(e1)
+    last = eng.download(dout, params) if a.dump_outputs and rank == 0 else None     # outputs of the last timed step
     launches = eng.launch_count() * a.steps
     # per-stage device times (events inside the library, same stream), averaged over K more steps
     stage_acc = {}
@@ -430,6 +472,8 @@ def run_b200(a):
         if world > 1:
             dist.destroy_process_group()
         return
+    if a.dump_outputs:
+        dump_outputs(last, a.dump_outputs)
 
     peaks_path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(peaks_path):

@@ -230,6 +230,47 @@ int mgatk_pileup_host_submit(mgatk_handle *h, const mgatk_params *params, const 
                              const mgatk_outputs *out_host, int64_t *ticket);
 int mgatk_pileup_host_wait(mgatk_handle *h, int64_t ticket);
 
+/* ---- variant statistics (DESIGN §8, "Variant statistics") ------------------
+ * A cross-cell reduction over the filtered planes of a result, for the heteroplasmy statistics of Signac's
+ * IdentifyVariants. Every count is exact: a plane entry of 65535 takes its value from the overflow list
+ * (stats->n_overflow entries of result->overflow; an entry of 65535 without a list entry is 65535). The reference
+ * allele ref[p] is the vote of result->base_totals: the first of A,C,G,T with the largest total, N when none is
+ * positive. For every position p with ref[p] != N and every b in A,C,G,T other than ref[p] there is one variant
+ * p ref>b; per selected cell, f / r are the b forward / reverse counts, a = f + r and d the coverage entry.
+ * out is laid out [P][4] by alt letter; the slot alt == ref and every slot of an N position have valid = 0 and all
+ * sums 0. */
+typedef struct mgatk_variant_sums {
+    uint64_t sum_fwd, sum_rev, sum_cov;  /* sum of f, r, d over the selected cells                                  */
+    uint64_t sum_ff, sum_rr, sum_fr;     /* over the cells with a > 0: sum of f*f, r*r, f*r                          */
+    uint64_t max_alt, max_cov;           /* (a, d) of the largest a/d over cells with d > 0 (exact cross-multiplied
+                                            compare; ties keep the lowest cell index); 0, 0 when no cell has d > 0   */
+    double   dev_sum, dev_sq;            /* sum of u and u*u, u = a/d - mean for cells with d >= L, else 0;
+                                            mean = (sum_fwd + sum_rev) / sum_cov, 0 when sum_cov = 0                 */
+    uint32_t n_covered;                  /* cells with d > 0                                                         */
+    uint32_t n_detected;                 /* cells with a > 0 (= the cells of sum_ff, sum_rr, sum_fr)                 */
+    uint32_t n_conf_detected;            /* cells with f >= 2 and r >= 2                                             */
+    uint32_t n_strand;                   /* cells with a > 0 (the n of the strand correlation)                       */
+    uint32_t n_over[4];                  /* cells with d > 0 and 100 a >= k d, k = 5, 10, 20, 95                     */
+    uint32_t n_low;                      /* cells with d < L (L = low_coverage_threshold)                            */
+    int32_t  ref;                        /* reference allele 0..3 = A,C,G,T; -1 = N                                  */
+    int32_t  valid;                      /* 1: a variant; 0: alt == ref or ref = N                                    */
+    int32_t  reserved;                   /* 0 */
+} mgatk_variant_sums;                    /* 128 bytes */
+
+/* Variant sums of the result `result_dev` (planes [n_cells][11][MGATK_POS_PAD(P)], stats, overflow, base_totals; all
+ * device pointers) over the cells with cell_mask_dev[c] != 0 (u8[n_cells]; NULL = all cells), into
+ * out_dev[P][4]. Integer fields do not depend on the launch configuration; dev_sum / dev_sq are reduced in a fixed
+ * order, so a call gives the same bits every time. Enqueues on `stream`; the overflow lookup table lives in the
+ * handle, so calls on one handle must be ordered (one stream). */
+int mgatk_variant_stats_device(mgatk_handle *h, const mgatk_params *params, const mgatk_outputs *result_dev,
+                               const uint8_t *cell_mask_dev, int32_t low_coverage_threshold,
+                               mgatk_variant_sums *out_dev, void *stream);
+/* Exact per-cell counts of n_variants variants (variants_dev: int32 pos * 4 + alt, pos in [0, P), alt 0..3 = A,C,G,T)
+ * for every cell: out_dev[n_variants][3][n_cells] = alt forward, alt reverse, coverage. An id outside [0, 4 P) gives
+ * rows of zeros. Enqueues on `stream`; same handle rule as above. */
+int mgatk_variant_cells_device(mgatk_handle *h, const mgatk_params *params, const mgatk_outputs *result_dev,
+                               const int32_t *variants_dev, int32_t n_variants, uint32_t *out_dev, void *stream);
+
 /* number of kernel launches issued by the last mgatk_pileup_* call on this handle */
 int64_t mgatk_last_launch_count(const mgatk_handle *h);
 

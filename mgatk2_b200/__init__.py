@@ -13,7 +13,8 @@ __all__ = ["ReadBatch", "PipelineConfig", "QualityThresholds", "DeduplicationCon
            "MgatkError", "InvalidInputError", "ProcessingError", "BAMReadError", "NoBarcodeTagsError",
            "PileupKernelError", "BAMReader", "CellProcessor", "process_barcode_worker", "PileupGenerator",
            "PileupEngine", "MtDNAPipeline", "run_pipeline", "load_singlecell_csv", "extract_barcodes_from_bam",
-           "DenseTextWriter", "DenseHDF5Writer", "report_inputs"]
+           "DenseTextWriter", "DenseHDF5Writer", "report_inputs",
+           "VARIANT_SUMS_DTYPE", "variant_sums", "finalize", "call_variants", "variant_cells"]
 
 
 def __getattr__(name):        # heavy pieces (ctypes library, torch) load on first use
@@ -38,6 +39,9 @@ def __getattr__(name):        # heavy pieces (ctypes library, torch) load on fir
     if name == "report_inputs":
         from .report import report_inputs
         return report_inputs
+    if name in ("VARIANT_SUMS_DTYPE", "variant_sums", "finalize", "call_variants", "variant_cells"):
+        from . import variants
+        return getattr(variants, name)
     if name == "PileupEngine":
         from .engine import PileupEngine
         return PileupEngine

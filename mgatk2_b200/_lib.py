@@ -15,6 +15,7 @@ EXPORTS = (
     "mgatk_workspace_bytes", "mgatk_pileup_device", "mgatk_check_stats", "mgatk_pileup_host",
     "mgatk_filter_strand_bias_device", "mgatk_filter_strand_bias_u32_device", "mgatk_stream_begin_device", "mgatk_stream_finish_device",
     "mgatk_last_launch_count", "mgatk_last_stage_times", "mgatk_pileup_host_submit", "mgatk_pileup_host_wait",
+    "mgatk_variant_stats_device", "mgatk_variant_cells_device",
 )
 
 N_PLANES = 11
@@ -37,6 +38,17 @@ class OutputsC(ctypes.Structure):
     _fields_ = [("planes", ctypes.c_void_p), ("cell_qc", ctypes.c_void_p), ("stats", ctypes.c_void_p),
                 ("base_totals", ctypes.c_void_p), ("overflow", ctypes.c_void_p),
                 ("overflow_capacity", ctypes.c_int64)]
+
+
+class VariantSumsC(ctypes.Structure):
+    """mgatk_variant_sums (128 bytes)."""
+    _fields_ = [("sum_fwd", ctypes.c_uint64), ("sum_rev", ctypes.c_uint64), ("sum_cov", ctypes.c_uint64),
+                ("sum_ff", ctypes.c_uint64), ("sum_rr", ctypes.c_uint64), ("sum_fr", ctypes.c_uint64),
+                ("max_alt", ctypes.c_uint64), ("max_cov", ctypes.c_uint64),
+                ("dev_sum", ctypes.c_double), ("dev_sq", ctypes.c_double),
+                ("n_covered", ctypes.c_uint32), ("n_detected", ctypes.c_uint32), ("n_conf_detected", ctypes.c_uint32),
+                ("n_strand", ctypes.c_uint32), ("n_over", ctypes.c_uint32 * 4), ("n_low", ctypes.c_uint32),
+                ("ref", ctypes.c_int32), ("valid", ctypes.c_int32), ("reserved", ctypes.c_int32)]
 
 
 class ExtensionMissingError(RuntimeError):
@@ -82,6 +94,10 @@ def load():
     lib.mgatk_last_launch_count.argtypes = [ctypes.c_void_p]
     lib.mgatk_last_stage_times.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_char_p),
                                            ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_int)]
+    lib.mgatk_variant_stats_device.argtypes = [ctypes.c_void_p, ctypes.POINTER(ParamsC), ctypes.POINTER(OutputsC),
+                                               ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p]
+    lib.mgatk_variant_cells_device.argtypes = [ctypes.c_void_p, ctypes.POINTER(ParamsC), ctypes.POINTER(OutputsC),
+                                               ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p]
     if lib.mgatk_abi_version() != ABI_VERSION:
         raise ExtensionMissingError(f"ABI mismatch: library {lib.mgatk_abi_version()}, binding {ABI_VERSION}")
     _lib = lib

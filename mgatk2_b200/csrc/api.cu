@@ -12,6 +12,7 @@
 #include "dedup.cuh"
 #include "pileup.cuh"
 #include "epilogue.cuh"
+#include "variants.cuh"
 
 using namespace mgatk;
 
@@ -129,6 +130,8 @@ struct mgatk_handle {
     // side stream of the overflow-list kernel (runs next to the main pileup kernel): fork / join events
     cudaStream_t side = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+    // variant statistics: hash table of the overflow list of the result being reduced
+    DevBuf var_table;
 };
 
 namespace {
@@ -483,6 +486,30 @@ int filter_planes(mgatk_handle *h, T *planes_dev, int32_t n_cells, int32_t mito_
     return MGATK_OK;
 }
 
+// checks shared by the variant entries; builds the overflow lookup table of `o` on `s` (*table: nullptr without a list)
+int variant_prepare(mgatk_handle *h, const mgatk_params *p, const mgatk_outputs *o, cudaStream_t s, const OvfSlot **table) {
+    *table = nullptr;
+    if (!p || !o) return fail(h, MGATK_ERR_BAD_ARG, "null argument");
+    if (p->n_cells < 0 || p->mito_length <= 0 || o->overflow_capacity < 0) return fail(h, MGATK_ERR_BAD_ARG, "negative size");
+    if (p->mito_length >= (1 << 24)) return fail(h, MGATK_ERR_RANGE, "mito_length must be below 2^24");
+    if (!o->stats || !o->base_totals || (p->n_cells > 0 && !o->planes)) return fail(h, MGATK_ERR_BAD_ARG, "null result array");
+    if (o->overflow_capacity > 0 && !o->overflow) return fail(h, MGATK_ERR_BAD_ARG, "null overflow list");
+    if (o->overflow_capacity > (int64_t)1 << 30) return fail(h, MGATK_ERR_RANGE, "overflow_capacity above 2^30");
+    CU(cudaSetDevice(h->device));
+    if (o->overflow_capacity == 0 || p->n_cells == 0) return MGATK_OK;
+    const u64 slots = ovf_table_slots((u64)o->overflow_capacity);
+    int rc = ensure(h, h->var_table, (size_t)slots * sizeof(OvfSlot));
+    if (rc) return rc;
+    OvfSlot *t = (OvfSlot *)h->var_table.p;
+    const unsigned clear_blocks = (unsigned)((slots + 255) / 256 < 1024 ? (slots + 255) / 256 : 1024);
+    const unsigned insert_blocks = (unsigned)((o->overflow_capacity + 255) / 256 < 1024 ? (o->overflow_capacity + 255) / 256 : 1024);
+    k_ovf_clear<<<clear_blocks, 256, 0, s>>>(t, o->stats, o->overflow_capacity);
+    k_ovf_insert<<<insert_blocks, 256, 0, s>>>(t, o->overflow, o->stats, o->overflow_capacity);
+    CU(cudaGetLastError());
+    *table = t;
+    return MGATK_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -532,6 +559,7 @@ int mgatk_destroy(mgatk_handle *h) {
     if (h->ws.p) cudaFree(h->ws.p);
     if (h->deep_planes.p) cudaFree(h->deep_planes.p);
     if (h->deep_map.p) cudaFree(h->deep_map.p);
+    if (h->var_table.p) cudaFree(h->var_table.p);
     if (h->s_h2d) { cudaStreamDestroy(h->s_h2d); cudaStreamDestroy(h->s_d2h); }
     if (h->events_ready) for (int i = 0; i <= kMaxStages; i++) cudaEventDestroy(h->ev[i]);
     if (h->stream) cudaStreamDestroy(h->stream);
@@ -728,6 +756,43 @@ int mgatk_pileup_host(mgatk_handle *h, const mgatk_params *p, const mgatk_batch 
     int rc = mgatk_pileup_host_submit(h, p, b, o, &ticket);
     if (rc) return rc;
     return mgatk_pileup_host_wait(h, ticket);
+}
+
+int mgatk_variant_stats_device(mgatk_handle *h, const mgatk_params *p, const mgatk_outputs *o, const uint8_t *cell_mask_dev,
+                               int32_t low_coverage_threshold, mgatk_variant_sums *out_dev, void *stream) {
+    if (!h) return MGATK_ERR_BAD_ARG;
+    h->err.clear();
+    if (!out_dev) return fail(h, MGATK_ERR_BAD_ARG, "null output array");
+    if (low_coverage_threshold < 1) return fail(h, MGATK_ERR_BAD_ARG, "low_coverage_threshold must be >= 1");
+    cudaStream_t s = (cudaStream_t)stream;
+    const OvfSlot *table = nullptr;
+    int rc = variant_prepare(h, p, o, s, &table);
+    if (rc) return rc;
+    VarArgs a;
+    a.planes = o->planes; a.stats = o->stats; a.totals = o->base_totals; a.table = table; a.ovf_cap = o->overflow_capacity;
+    a.mask = cell_mask_dev; a.C = p->n_cells; a.P = p->mito_length; a.ppad = (int)MGATK_POS_PAD(p->mito_length);
+    a.low = (u32)low_coverage_threshold; a.out = out_dev;
+    k_variant_stats<<<(unsigned)((a.P + kVarTile - 1) / kVarTile), kVarWarps * 32, 0, s>>>(a);
+    CU(cudaGetLastError());
+    return MGATK_OK;
+}
+
+int mgatk_variant_cells_device(mgatk_handle *h, const mgatk_params *p, const mgatk_outputs *o, const int32_t *variants_dev,
+                               int32_t n_variants, uint32_t *out_dev, void *stream) {
+    if (!h) return MGATK_ERR_BAD_ARG;
+    h->err.clear();
+    if (n_variants < 0) return fail(h, MGATK_ERR_BAD_ARG, "negative n_variants");
+    if (n_variants > 0 && (!variants_dev || !out_dev)) return fail(h, MGATK_ERR_BAD_ARG, "null variant or output array");
+    cudaStream_t s = (cudaStream_t)stream;
+    const OvfSlot *table = nullptr;
+    int rc = variant_prepare(h, p, o, s, &table);
+    if (rc) return rc;
+    if (n_variants == 0 || p->n_cells == 0) return MGATK_OK;
+    dim3 grid((unsigned)((p->n_cells + 255) / 256), (unsigned)(n_variants < 65535 ? n_variants : 65535));
+    k_variant_cells<<<grid, 256, 0, s>>>(o->planes, table, o->stats, o->overflow_capacity, variants_dev, n_variants, p->n_cells,
+                                         p->mito_length, (int)MGATK_POS_PAD(p->mito_length), out_dev);
+    CU(cudaGetLastError());
+    return MGATK_OK;
 }
 
 int64_t mgatk_last_launch_count(const mgatk_handle *h) { return h ? h->launches : 0; }

@@ -38,7 +38,10 @@ class MtDNAPipeline:
     def __init__(self, bam_path: str, barcodes: list, output_dir, config: PipelineConfig | None = None,
                  output_format: str = "standard", barcode_metadata=None, sample_name: str = "mgatk2",
                  report_title: str | None = None, report_subtitle: str | None = None, working_directory: str | None = None,
-                 device: int = 0, devices: list | None = None, max_batch_records: int | None = None):
+                 device: int = 0, devices: list | None = None, max_batch_records: int | None = None,
+                 call_variants: bool = False):
+        """`call_variants=True` adds `output/variant_stats.tsv.gz` and `output/variant_cells.tsv.gz` (variants.py) after
+        the reference's outputs, which stay as they are."""
         self.bam_path = Path(bam_path)
         self.barcodes = set(barcodes)
         self.barcode_list = list(barcodes)
@@ -50,6 +53,7 @@ class MtDNAPipeline:
         self.devices = list(devices) if devices else [device]      # GPUs of this box; the cells are split between them
         self.device = self.devices[0]
         self.max_batch_records = max_batch_records                  # larger contigs are streamed in parts (dispatch.py)
+        self.call_variants = bool(call_variants)
         if not self.bam_path.exists():
             raise InvalidInputError(f"BAM file not found: {bam_path}")
         from .bamio import BamFile, pick_mito_contig
@@ -87,6 +91,12 @@ class MtDNAPipeline:
             return {}
         qc_dir = self.output_dir / "qc"
         writer.finalize(qc_dir)
+        if self.call_variants:
+            from .pileup import get_engine
+            from .variants import write_variant_files
+            called = write_variant_files(reads_by_barcode.result, self.barcode_list, self.output_dir / "output",
+                                         engine=get_engine(self.device))
+            logger.info("%d variants called", len(called))
         self.timings = dict(getattr(reader, "timings", {}), write_s=time.time() - t_write, total_s=time.time() - start)
         c = self.config
         write_run_summary({                                               # analysis/qc.py:68-93
@@ -108,13 +118,14 @@ class MtDNAPipeline:
 
 def run_pipeline(bam_path: str, output_dir: str, barcode_file: str | None = None, min_barcode_reads: int = 10,
                  barcode_tag: str = "CB", mito_chr: str = "chrM", output_format: str = "standard", device: int = 0,
-                 devices: list | None = None, max_batch_records: int | None = None, **config_kwargs) -> dict:
+                 devices: list | None = None, max_batch_records: int | None = None, call_variants: bool = False,
+                 **config_kwargs) -> dict:
     """core.pipeline.run_pipeline (pipeline.py:184-270): whitelist from file / singlecell.csv / the BAM itself, then
-    `MtDNAPipeline.run()`. `config_kwargs` are `PipelineConfig` keywords (min_baseq, min_mapq, max_strand_bias,
+    `MtDNAPipeline.run()` (`call_variants`: as there). `config_kwargs` are `PipelineConfig` keywords (min_baseq, min_mapq, max_strand_bias,
     skip_deduplication, use_fragment_length_dedup, min_reads_per_cell, ...)."""
     barcodes, metadata = load_barcodes(barcode_file, bam_path, barcode_tag=barcode_tag, mito_chr=mito_chr,
                                        min_barcode_reads=min_barcode_reads)
     config = PipelineConfig(barcode_tag=barcode_tag, mito_chr=mito_chr, **config_kwargs)
     return MtDNAPipeline(bam_path, barcodes, Path(output_dir), config, output_format=output_format,
                          barcode_metadata=metadata, device=device, devices=devices,
-                         max_batch_records=max_batch_records).run()
+                         max_batch_records=max_batch_records, call_variants=call_variants).run()

@@ -226,13 +226,13 @@ int launch_scatter(mgatk_handle *h, cudaStream_t s, const ScatterArgs &a) {
 
 constexpr int kChrMPpad = (int)MGATK_POS_PAD(16569);    // the plane pitch of chrM is compiled in
 
-template <bool kCompact, int kPpad>
+template <bool kCompact, int kPpad, bool kAcc>
 int launch_pileup_t(mgatk_handle *h, cudaStream_t s, const PileupArgs &a, const PileupArgs &a_big, int stage_bytes) {
-    const size_t smem_main = (size_t)PileupStages<kCompact>::value * stage_bytes, smem_big = (size_t)stage_bytes;
-    CU(cudaFuncSetAttribute(k_pileup_main<kCompact, kPpad>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_main));
+    const size_t smem_main = (size_t)PileupStages<kCompact>::value * (stage_bytes + range_table_bytes(a.ppad)), smem_big = (size_t)stage_bytes;
+    CU(cudaFuncSetAttribute(k_pileup_main<kCompact, kPpad, kAcc>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_main));
     CU(cudaFuncSetAttribute(k_pileup_big<kCompact, kPpad>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_big));
     int per_sm = 0, per_sm_big = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_pileup_main<kCompact, kPpad>, kThreads + 32, smem_main));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_pileup_main<kCompact, kPpad, kAcc>, kThreads + 32, smem_main));
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_big, k_pileup_big<kCompact, kPpad>, kThreads, smem_big));
     if (per_sm < 1) per_sm = 1;
     if (per_sm_big < 1) per_sm_big = 1;
@@ -247,17 +247,25 @@ int launch_pileup_t(mgatk_handle *h, cudaStream_t s, const PileupArgs &a, const 
     CU(cudaStreamWaitEvent(h->side, h->ev_fork, 0));
     k_pileup_big<kCompact, kPpad><<<h->sm_count * per_sm_big, kThreads, smem_big, h->side>>>(a_big);
     CU(cudaEventRecord(h->ev_join, h->side));
-    k_pileup_main<kCompact, kPpad><<<h->sm_count * per_sm, kThreads + 32, smem_main, s>>>(a, stage_bytes);   // persistent CTAs pulling units
+    k_pileup_main<kCompact, kPpad, kAcc><<<h->sm_count * per_sm, kThreads + 32, smem_main, s>>>(a, stage_bytes);   // persistent CTAs pulling units
     CU(cudaStreamWaitEvent(s, h->ev_join, 0));
     h->launches += 2;
     CU(cudaGetLastError());
     return MGATK_OK;
 }
 
+template <int kPpad, bool kAcc>
+int launch_pileup_p(mgatk_handle *h, cudaStream_t s, bool compact, const PileupArgs &a, const PileupArgs &a_big, int stage_bytes) {
+    return compact ? launch_pileup_t<true, kPpad, kAcc>(h, s, a, a_big, stage_bytes) : launch_pileup_t<false, kPpad, kAcc>(h, s, a, a_big, stage_bytes);
+}
+
+// the instance of the main kernel: slot layout, chrM's plane pitch or any other, streaming (accumulate) or not
 int launch_pileup(mgatk_handle *h, cudaStream_t s, bool compact, const PileupArgs &a, const PileupArgs &a_big, int stage_bytes) {
     if (a.ppad == kChrMPpad)
-        return compact ? launch_pileup_t<true, kChrMPpad>(h, s, a, a_big, stage_bytes) : launch_pileup_t<false, kChrMPpad>(h, s, a, a_big, stage_bytes);
-    return compact ? launch_pileup_t<true, 0>(h, s, a, a_big, stage_bytes) : launch_pileup_t<false, 0>(h, s, a, a_big, stage_bytes);
+        return a.accumulate ? launch_pileup_p<kChrMPpad, true>(h, s, compact, a, a_big, stage_bytes)
+                            : launch_pileup_p<kChrMPpad, false>(h, s, compact, a, a_big, stage_bytes);
+    return a.accumulate ? launch_pileup_p<0, true>(h, s, compact, a, a_big, stage_bytes)
+                        : launch_pileup_p<0, false>(h, s, compact, a, a_big, stage_bytes);
 }
 
 int validate(mgatk_handle *h, const mgatk_params *p, const mgatk_batch *b, const mgatk_outputs *o) {

@@ -103,7 +103,7 @@ k_stream_finish(PileupArgs a, int n_cells, int min_reads) {
             if (set >= 0 && !dead) cnt[k] += a.deep_planes[((size_t)set * 10 + k) * a.ppad + 32 * ch + lane] << 16;
         }
         u64 sum = 0; u32 covered = 0, maxd = 0;
-        finish_chunk<0>(a, cell, 32 * ch, lane, cnt, sum, covered, maxd);
+        finish_chunk<0, false>(a, cell, 32 * ch, lane, cnt, sum, covered, maxd);
         if (__any_sync(kFull, covered != 0)) {
             u64 tot = sum;
             for (int o = 16; o; o >>= 1) tot += __shfl_xor_sync(kFull, tot, o);

@@ -3,14 +3,16 @@
 // (pileup.py:128-154) and the per-cell depth statistics, planes written once.
 //
 //   k_plan_scan / k_plan_units   cut every cell into position tiles ("units") of bounded read count
-//   k_pileup_main                persistent CTAs, warp-specialised: a producer warp pulls units from a global counter and
-//                                streams each unit's slots into shared memory with ONE bulk asynchronous copy (TMA),
-//                                two units in flight per CTA, full / empty mbarriers; the eight consumer warps take
-//                                chunks of 32 positions and never meet at a CTA barrier
+//   k_pileup_main                persistent CTAs, warp-specialised: a producer warp pulls units from a global counter,
+//                                streams each unit's slots into shared memory with ONE bulk asynchronous copy (TMA)
+//                                (full mbarrier), then builds the unit's table of candidate ranges per chunk (ready
+//                                mbarrier); three units in flight per CTA; the eight consumer warps take chunks of 32
+//                                positions, release a stage on its empty mbarrier and never meet at a CTA barrier
 //   k_pileup_big                 the rare units that do not fit a stage (hot spots, piles beyond 65535): sub-tiles and
 //                                batches, plain loads, CTA barriers
 //
-// Counting a chunk: the candidate reads are those starting in (chunk - extent, chunk + 32); 32 candidates at a time,
+// Counting a chunk: the candidate reads are those starting in (chunk - extent, chunk + 32), a range of the unit's slots
+// read from the table (k_pileup_main) or found by a 32-way search (k_pileup_big); 32 candidates at a time,
 // one per lane: the 32-bit window of the read's three planes at offset chunk - start; a 32x32 bit transpose across the
 // warp turns "lane = read" into "lane = position" for the four bit matrices of the round (V, B0, B1 and the Tn5 sites;
 // one or two transposes when the candidates fit 8 or 16 lanes), and one LOP3 + popcount per base and strand adds up the
@@ -204,17 +206,17 @@ __device__ __forceinline__ int deep_set_of(const PileupArgs &a, int cell, int la
 }
 
 // The counts of a chunk are final: strand-bias filter, coverage, Tn5 gating (pileup.py:128-154), depth
-// statistics, saturation (writers.py:205-218) and the one write of the 11 planes.
-template <int kPpad>
+// statistics, saturation (writers.py:205-218) and the one write of the 11 planes. kAcc: a.accumulate, compiled in.
+template <int kPpad, bool kAcc>
 __device__ __forceinline__ void finish_chunk(const PileupArgs &a, int cell, int c0, int lane, u32 (&cnt)[10],
                                              u64 &sum, u32 &covered, u32 &maxd) {
     const int ppad = kPpad ? kPpad : a.ppad;             // compile-time plane pitch: the 11 stores share one address
     const int p = c0 + lane;
-    if (p >= a.P) {                                  // pileup.py:58 end_refpos = min(.., mito_length): padding stays zero
-#pragma unroll
-        for (int k = 0; k < 10; k++) cnt[k] = 0;
+    if (c0 + 32 > a.P) {                             // the contig's last chunk only (warp-uniform)
+#pragma unroll                                       // pileup.py:58 end_refpos = min(.., mito_length): padding stays zero
+        for (int k = 0; k < 10; k++) cnt[k] = p >= a.P ? 0u : cnt[k];
     }
-    if (a.accumulate) {                              // streamed batches: raw counts add up in the planes; filters, coverage
+    if (kAcc) {                                      // streamed batches: raw counts add up in the planes; filters, coverage
         uint16_t *acc = a.planes + (size_t)cell * MGATK_N_PLANES * ppad + p;      // and statistics come in k_stream_finish
         u32 v[10], wraps = 0u;
 #pragma unroll
@@ -280,6 +282,12 @@ __device__ __forceinline__ void finish_chunk(const PileupArgs &a, int cell, int 
     uint16_t *out = a.planes + (size_t)cell * MGATK_N_PLANES * ppad + p;
 #pragma unroll
     for (int pl = 0; pl < MGATK_N_PLANES; pl++) out[(size_t)pl * ppad] = (uint16_t)vals[pl];
+}
+template <int kPpad>
+__device__ __forceinline__ void finish_chunk_rt(const PileupArgs &a, int cell, int c0, int lane, u32 (&cnt)[10],
+                                                u64 &sum, u32 &covered, u32 &maxd) {
+    if (a.accumulate) finish_chunk<kPpad, true>(a, cell, c0, lane, cnt, sum, covered, maxd);
+    else finish_chunk<kPpad, false>(a, cell, c0, lane, cnt, sum, covered, maxd);
 }
 
 // Per-base form of one aligned block for an indirect read (no planes in its slot): chunk bits [pa, pa + span)
@@ -397,54 +405,80 @@ __device__ __forceinline__ int first_above(u32 addr, u32 stride, int n, int key,
     return lo;
 }
 
-// Counts of the 32 positions from c0 out of the n slots at `addr` (shared memory), part `part` of `nparts` of the
-// candidates: lane = position on return. `first` = first slot that can reach the chunk.
+// One round of a chunk's counting: the nc candidates (1 <= nc <= 32) from slot r of the slots at `addr` (shared memory),
+// one per lane, are added to the counts of the 32 positions from c0 (lane = position).
 template <bool kCompact>
-__device__ __forceinline__ void count_chunk(const PileupArgs &a, u32 addr, int n, int first, int c0, int part, int nparts, int lane,
+__device__ __forceinline__ void count_round(const PileupArgs &a, u32 addr, int r, int nc, int c0, int lane,
                                             const TransposeConst &tc, u32 (&cnt)[10]) {
-    const int c1 = c0 + 32;
-    const int skip_le = c0 - a.extent;               // reads starting at or before this cannot reach the chunk
-    const u32 stride = (u32)a.slot_bytes;
-    for (int r = first + 32 * part; r < n; r += 32 * nparts) {
-        const int j = r + lane;
+    u32 pv = 0u, p0 = 0u, p1 = 0u, m5 = 0u;                  // planes of this read inside the chunk: valid base, code bits, Tn5 site
+    int strand = 0;
+    if (lane < nc) {
         SlotView<kCompact> sv;
-        const u32 s = addr + (u32)j * stride;
-        int pos = 0x7fffffff;
-        if (j < n) { sv.load(s); pos = sv.pos(); }
-        const u32 m_after = __ballot_sync(kFull, pos >= c1);
-        const bool cand = pos < c1 && pos > skip_le;                              // implies j < n
-        const u32 cands = __ballot_sync(kFull, cand);
-        if (cands) {
-            u32 pv = 0u, p0 = 0u, p1 = 0u, m5 = 0u;          // planes of this read inside the chunk: valid base, code bits, Tn5 site
-            int strand = 0;
-            if (cand) {
-                strand = (sv.meta() & SM_STRAND) ? 1 : 0;
-                // Tn5 site (pileup.py:43-50): reverse = start + len(SEQ) - 1, forward = start
-                const int t5 = strand ? pos + sv.tn5off() : pos;
-                if ((u32)(t5 - c0) < 32u && t5 < a.P) m5 = 1u << (t5 - c0);
-                sv.window(a, s, c0 - pos, pv, p0, p1);
-            }
-            // lane = read -> lane = position. The four bit matrices of a round (V, B0, B1, Tn5; rows = reads) share one
-            // 32x32 transpose when its candidates sit in lanes 0..7 (one matrix per byte), two when they sit in lanes
-            // 0..15; forward and reverse reads are counted apart (pileup.py:88)
-            const u32 rev = __ballot_sync(kFull, cand && strand);
-            u32 v, b0, b1, t5;
-            if (cands <= 0xffu) {
-                const int src = lane & 7;
-                const u32 s0 = __shfl_sync(kFull, p0, src), s1 = __shfl_sync(kFull, p1, src), s5 = __shfl_sync(kFull, m5, src);
-                quarter_columns(warp_transpose(quarter_row(lane, pv, s0, s1, s5), tc), v, b0, b1, t5);
-            } else if (cands <= 0xffffu) {
-                const u32 s0 = __shfl_xor_sync(kFull, p0, 16), s5 = __shfl_xor_sync(kFull, m5, 16);
-                const u32 ta = warp_transpose(half_row(lane, pv, s0), tc);
-                const u32 tb = warp_transpose(half_row(lane, p1, s5), tc);
-                half_columns(ta, tb, v, b0, b1, t5);
-            } else {
-                v = warp_transpose(pv, tc); b0 = warp_transpose(p0, tc); b1 = warp_transpose(p1, tc); t5 = warp_transpose(m5, tc);
-            }
-            count_columns(v, b0, b1, t5, rev, cnt);
-        }
-        if (m_after) break;
+        const u32 s = addr + (u32)(r + lane) * (kCompact ? 32u : (u32)a.slot_bytes);
+        sv.load(s);
+        const int pos = sv.pos();
+        strand = (sv.meta() & SM_STRAND) ? 1 : 0;
+        // Tn5 site (pileup.py:43-50): reverse = start + len(SEQ) - 1, forward = start
+        const int t5 = strand ? pos + sv.tn5off() : pos;
+        if ((u32)(t5 - c0) < 32u && t5 < a.P) m5 = 1u << (t5 - c0);
+        sv.window(a, s, c0 - pos, pv, p0, p1);
     }
+    // lane = read -> lane = position. The four bit matrices of a round (V, B0, B1, Tn5; rows = reads) share one 32x32
+    // transpose when there are at most 8 candidates (one matrix per byte), two when there are at most 16; forward and
+    // reverse reads are counted apart (pileup.py:88)
+    const u32 rev = __ballot_sync(kFull, strand);
+    u32 v, b0, b1, t5;
+    if (nc <= 8) {
+        const int src = lane & 7;
+        const u32 s0 = __shfl_sync(kFull, p0, src), s1 = __shfl_sync(kFull, p1, src), s5 = __shfl_sync(kFull, m5, src);
+        quarter_columns(warp_transpose(quarter_row(lane, pv, s0, s1, s5), tc), v, b0, b1, t5);
+    } else if (nc <= 16) {
+        const u32 s0 = __shfl_xor_sync(kFull, p0, 16), s5 = __shfl_xor_sync(kFull, m5, 16);
+        const u32 ta = warp_transpose(half_row(lane, pv, s0), tc);
+        const u32 tb = warp_transpose(half_row(lane, p1, s5), tc);
+        half_columns(ta, tb, v, b0, b1, t5);
+    } else {
+        v = warp_transpose(pv, tc); b0 = warp_transpose(p0, tc); b1 = warp_transpose(p1, tc); t5 = warp_transpose(m5, tc);
+    }
+    count_columns(v, b0, b1, t5, rev, cnt);
+}
+
+// Counts of the 32 positions from c0 out of the candidate slots [first, last) at `addr` (those starting in
+// (c0 - extent, c0 + 32)), part `part` of `nparts` of them: lane = position on return.
+template <bool kCompact>
+__device__ __forceinline__ void count_range(const PileupArgs &a, u32 addr, int first, int last, int c0, int part, int nparts,
+                                            int lane, const TransposeConst &tc, u32 (&cnt)[10]) {
+    for (int r = first + 32 * part; r < last; r += 32 * nparts) count_round<kCompact>(a, addr, r, min(last - r, 32), c0, lane, tc, cnt);
+}
+
+// Candidate ranges of every chunk of a unit whose n slots (sorted by start) sit at `addr`, built by one warp in one pass
+// over the slots: entry ch of the table at `tbl` holds the first slot starting after t0 + 32 ch - extent (low half) and
+// the first slot starting at or after t0 + 32 (ch + 1) (high half). Slot i fills the entries between its predecessor's
+// chunk bound and its own; the entries beyond the last slot's bounds (all of them in a unit without reads) take n,
+// written by all lanes.
+__device__ __forceinline__ void st_shared_u16(u32 a, int v) {
+    asm volatile("st.shared.u16 [%0], %1;" ::"r"(a), "h"((unsigned short)v) : "memory");
+}
+__device__ __forceinline__ void build_ranges(u32 addr, u32 stride, int n, int t0, int n_chunks, int extent, u32 tbl, int lane) {
+    const SharedMem smem;
+    int pf = -1, pb = 0;                                     // last low / high entry filled so far (high entries start at 1)
+    for (int i0 = 0; i0 < n; i0 += 32) {
+        const int i = i0 + lane;
+        int kf = pf, kb = pb;                                // lanes past the last slot fill nothing
+        if (i < n) {
+            const int x = (int)smem.ld32(addr + (u32)i * stride) - t0;
+            kf = max(min((x + extent - 1) >> 5, n_chunks - 1), -1);          // last chunk whose low entry is i (if any)
+            kb = max(min(x >> 5, n_chunks), 0);
+        }
+        int qf = __shfl_up_sync(kFull, kf, 1), qb = __shfl_up_sync(kFull, kb, 1);
+        if (lane == 0) { qf = pf; qb = pb; }
+        const int last = min(n - i0, 32) - 1;
+        pf = __shfl_sync(kFull, kf, last); pb = __shfl_sync(kFull, kb, last);
+        for (int c = qf + 1; c <= kf; c++) st_shared_u16(tbl + 4u * c, i);
+        for (int c = qb + 1; c <= kb; c++) st_shared_u16(tbl + 4u * c - 2u, i);
+    }
+    for (int c = pf + 1 + lane; c < n_chunks; c += 32) st_shared_u16(tbl + 4u * c, n);
+    for (int c = pb + 1 + lane; c <= n_chunks; c += 32) st_shared_u16(tbl + 4u * c - 2u, n);
 }
 
 // per-cell depth statistics of a finished unit (processors.py:36-39, writers.py:187-193): hardware warp reductions
@@ -481,88 +515,123 @@ __device__ __forceinline__ void unit_statistics(const PileupArgs &a, int cell, i
 // units in flight per CTA of the main kernel: a warp may run this far ahead of the slowest
 template <bool kCompact> struct PileupStages { static constexpr int value = kCompact ? MGATK_PILEUP_STAGES : MGATK_PILEUP_WIDE_STAGES; };
 
+// Candidate-range table of one stage of k_pileup_main: one entry per chunk of the unit. A unit spans at most ppad / 32
+// chunks; the table holds chrM's 518 (2 KB per stage: four CTAs per SM still fit), and on longer contigs a unit beyond
+// that searches its chunks' ranges instead.
+constexpr int kMaxRangeChunks = (int)MGATK_POS_PAD(16569) / 32;
+__host__ __device__ inline int range_table_chunks(int ppad) { return ppad / 32 < kMaxRangeChunks ? ppad / 32 : kMaxRangeChunks; }
+__host__ __device__ inline int range_table_bytes(int ppad) { return (4 * range_table_chunks(ppad) + 15) / 16 * 16; }
+
+// The next unit with at least one chunk from the global counter (lane 0); cell -1 when there is none left.
+__device__ __forceinline__ Unit claim_unit(const PileupArgs &a, int n_units) {
+    Unit un;
+    for (;;) {
+        const int u = atomicAdd(a.work_counter, 1);
+        if (u >= n_units) { un.cell = -1; un.t0 = un.t1 = un.rbeg = un.rend = 0; return un; }
+        un = a.units[u];
+        if (un.t1 - un.t0 >= 32) return un;                  // else an empty tile (its reads belong to the tile before, or to k_pileup_big)
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
-// Main kernel: every unit fits one stage. Warp kWarpsPerCta is the producer: unit index from the global counter, the
-// unit descriptor into the stage, one bulk copy of the unit's slots (contiguous in the compacted array) signalled on
-// the stage's `full` barrier. Consumer warps wait for `full`, count their chunks (round-robin) straight out of the
-// stage, release it on `empty` (one arrival per warp) and move on to the other stage: no CTA-wide barrier, a slow warp
-// only holds back the refill of its own stage.
+// Main kernel: every unit fits one stage. Warp kWarpsPerCta is the producer: the unit descriptor into the stage, one
+// bulk copy of the unit's slots (contiguous in the compacted array) signalled on the stage's `full` barrier. Once the
+// slots have landed the producer builds the stage's candidate-range table (build_ranges) and signals `ready`. Consumer
+// warps wait for `ready`, take chunks as they come for them, count each from its table entry straight out of the stage,
+// release the stage on `empty` (one arrival per warp) and move on to the next: no CTA-wide barrier, a slow warp only
+// holds back the refill of its own stage.
+// kAcc: streaming (a.accumulate), compiled in.
 // ---------------------------------------------------------------------------------------------
-template <bool kCompact, int kPpad>
+template <bool kCompact, int kPpad, bool kAcc>
 __global__ void __launch_bounds__(kThreads + 32, kCompact ? MGATK_PILEUP_CTAS : 3)     // wide slots: the walk over plane groups needs the registers
 k_pileup_main(PileupArgs a, int stage_bytes) {
     constexpr int kStages = PileupStages<kCompact>::value;
-    extern __shared__ __align__(128) uint8_t dyn[];          // [kStages][stage_bytes]
-    __shared__ __align__(8) u64 s_full[kStages], s_empty[kStages];
+    extern __shared__ __align__(128) uint8_t dyn[];          // [kStages][stage_bytes] slots, then [kStages][range_table_bytes] tables
+    __shared__ __align__(8) u64 s_full[kStages], s_ready[kStages], s_empty[kStages];
     __shared__ Unit s_unit[kStages];
     __shared__ int s_next[kStages];                          // next chunk of the stage's unit to hand out
     const int lane = lane_id(), wid = threadIdx.x >> 5;
     const u32 full0 = (u32)__cvta_generic_to_shared(&s_full[0]), empty0 = (u32)__cvta_generic_to_shared(&s_empty[0]);
+    const u32 ready0 = (u32)__cvta_generic_to_shared(&s_ready[0]);
     const u32 stage0 = (u32)__cvta_generic_to_shared(dyn);
+    const int table_chunks = range_table_chunks(kPpad ? kPpad : a.ppad);
+    constexpr bool kTableAlways = kPpad != 0 && kPpad / 32 <= kMaxRangeChunks;
+    const u32 table_bytes = (u32)range_table_bytes(kPpad ? kPpad : a.ppad);
+    const u32 table0 = stage0 + kStages * (u32)stage_bytes;
+    const u32 stride = kCompact ? 32u : (u32)a.slot_bytes;
     if (threadIdx.x == 0) {
-        for (int b = 0; b < kStages; b++) { mbar_init(full0 + 8u * b, 1); mbar_init(empty0 + 8u * b, kWarpsPerCta); }
+        for (int b = 0; b < kStages; b++) {
+            mbar_init(full0 + 8u * b, 1); mbar_init(ready0 + 8u * b, 32); mbar_init(empty0 + 8u * b, kWarpsPerCta);
+        }
         mbar_fence_init();
     }
     __syncthreads();
     if (wid == kWarpsPerCta) {                               // ---- producer ----
         const int n_units = *a.n_units;
         for (u32 k = 0;; k++) {
-            const u32 b = k % kStages;
+            const u32 b = k % kStages, ph = (k / kStages) & 1u;
             Unit un;
             if (lane == 0) {
-                if (k >= (u32)kStages) mbar_wait_sleepy(empty0 + 8u * b, ((k / kStages) - 1u) & 1u, 2000u);     // all consumer warps left the stage
-                for (;;) {
-                    const int u = atomicAdd(a.work_counter, 1);
-                    if (u >= n_units) { un.cell = -1; un.t0 = un.t1 = un.rbeg = un.rend = 0; break; }
-                    un = a.units[u];
-                    if (un.t1 - un.t0 >= 32) break;          // an empty tile (its reads belong to the tile before, or to k_pileup_big)
-                }
+                if (k >= (u32)kStages) mbar_wait_sleepy(empty0 + 8u * b, ph ^ 1u, 2000u);     // all consumer warps left the stage
+                // (claiming the unit before that wait, so that its descriptor load overlaps it, was measured slower:
+                // pileup 0.484 against 0.476 ms on C2)
+                un = claim_unit(a, n_units);
                 s_unit[b] = un;
                 s_next[b] = 0;
             }
-            un.cell = __shfl_sync(kFull, un.cell, 0); un.rbeg = __shfl_sync(kFull, un.rbeg, 0); un.rend = __shfl_sync(kFull, un.rend, 0);
+            un.cell = __shfl_sync(kFull, un.cell, 0); un.t0 = __shfl_sync(kFull, un.t0, 0); un.t1 = __shfl_sync(kFull, un.t1, 0);
+            un.rbeg = __shfl_sync(kFull, un.rbeg, 0); un.rend = __shfl_sync(kFull, un.rend, 0);
             const int n = un.cell >= 0 ? un.rend - un.rbeg : 0;
-            const u32 bytes = (u32)n * (u32)a.slot_bytes;
+            const u32 bytes = (u32)n * stride;
             const u32 dst = stage0 + b * (u32)stage_bytes, bar = full0 + 8u * b;
             if (lane == 0) {
                 if (bytes) {                                 // the unit's slots are one contiguous range: one bulk copy
                     fence_proxy_async();
                     mbar_expect_tx(bar, bytes);
-                    bulk_load(dst, a.slots + (size_t)un.rbeg * a.slot_bytes, bytes, bar);
+                    bulk_load(dst, a.slots + (size_t)un.rbeg * stride, bytes, bar);
                 } else mbar_arrive(bar);
             }
+            const int n_chunks = (un.t1 - un.t0) >> 5;
+            if (un.cell >= 0 && n_chunks <= table_chunks) {
+                mbar_wait_sleepy(bar, ph, MGATK_PILEUP_HINT);
+                build_ranges(dst, stride, n, un.t0, n_chunks, a.extent, table0 + b * table_bytes, lane);
+            }
+            mbar_arrive(ready0 + 8u * b);                    // every lane: its own table entries are written
             if (un.cell < 0) break;
         }
         return;
     }
     // ---- consumers ----
     const TransposeConst tc = make_transpose_const(lane);
+    const SharedMem smem;
     for (u32 k = 0;; k++) {
-        const u32 b = k % kStages;
-#ifdef MGATK_PILEUP_SPIN
-        mbar_wait(full0 + 8u * b, (k / kStages) & 1u);
-#else
-        mbar_wait_sleepy(full0 + 8u * b, (k / kStages) & 1u, MGATK_PILEUP_HINT);
-#endif
+        const u32 b = k % kStages, ph = (k / kStages) & 1u;
+        mbar_wait_sleepy(ready0 + 8u * b, ph, MGATK_PILEUP_HINT);
         const Unit un = s_unit[b];
         if (un.cell < 0) break;
-        const u32 addr = stage0 + b * (u32)stage_bytes;
+        mbar_wait_sleepy(full0 + 8u * b, ph, MGATK_PILEUP_HINT);   // (complete already when the producer built the table)
+        const u32 addr = stage0 + b * (u32)stage_bytes, tbl = table0 + b * table_bytes;
         const int n = un.rend - un.rbeg, n_chunks = (un.t1 - un.t0) >> 5;
+        const bool table = kTableAlways || n_chunks <= table_chunks;
         u64 sum = 0; u32 covered = 0, maxd = 0;
-#ifndef MGATK_PILEUP_STATIC
         for (;;) {                                           // chunks are handed out as the warps come for them: a warp with a
             int ch = 0;                                      // crowded chunk (Tn5 hot spot) does not hold the others back
             if (lane == 0) ch = atomicAdd(&s_next[b], 1);    // (pileup 0.563 -> 0.539 ms on C2 against round-robin chunks)
             ch = __shfl_sync(kFull, ch, 0);
             if (ch >= n_chunks) break;
-#else
-        for (int ch = wid; ch < n_chunks; ch += kWarpsPerCta) {
-#endif
             const int c0 = un.t0 + 32 * ch;
             u32 cnt[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};   // 8 base x strand counters, Tn5 fwd / rev; lane = position
-            const int first = first_above(addr, (u32)a.slot_bytes, n, c0 - a.extent, lane);
-            count_chunk<kCompact>(a, addr, n, first, c0, 0, 1, lane, tc, cnt);
-            finish_chunk<kPpad>(a, un.cell, c0, lane, cnt, sum, covered, maxd);
+            int first, last;
+            if (table) {
+                const u32 e = smem.ld32(tbl + 4u * ch);
+                // (clamped: slots out of order, which the partition refuses, may leave entries unwritten)
+                last = min((int)(e >> 16), n); first = min((int)(e & 0xffffu), last);
+            } else {
+                first = first_above(addr, stride, n, c0 - a.extent, lane);
+                last = first_above(addr, stride, n, c0 + 31, lane);
+            }
+            count_range<kCompact>(a, addr, first, last, c0, 0, 1, lane, tc, cnt);
+            finish_chunk<kPpad, kAcc>(a, un.cell, c0, lane, cnt, sum, covered, maxd);
         }
         unit_statistics(a, un.cell, lane, sum, covered, maxd);
         __syncwarp();
@@ -655,12 +724,13 @@ k_pileup_big(PileupArgs a) {
                     const int c0 = un.t0 + 32 * chl;
                     u32 cnt[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
                     const int first = first_above(addr, (u32)a.slot_bytes, nb, c0 - a.extent, lane);
-                    count_chunk<kCompact>(a, addr, nb, first, c0, part, nparts, lane, tc, cnt);
+                    const int last = first_above(addr, (u32)a.slot_bytes, nb, c0 + 31, lane);
+                    count_range<kCompact>(a, addr, first, last, c0, part, nparts, lane, tc, cnt);
                     if (deep) {
 #pragma unroll
                         for (int k = 0; k < 10; k++) if (cnt[k]) atomicAdd(&s_acc[chl * kAccWords + k * 32 + lane], cnt[k]);
                     } else {
-                        finish_chunk<kPpad>(a, un.cell, c0, lane, cnt, sum, covered, maxd);
+                        finish_chunk_rt<kPpad>(a, un.cell, c0, lane, cnt, sum, covered, maxd);
                     }
                 }
                 rb += nb > 0 ? nb : 1;
@@ -671,7 +741,7 @@ k_pileup_big(PileupArgs a) {
                     u32 cnt[10];
 #pragma unroll
                     for (int k = 0; k < 10; k++) { cnt[k] = s_acc[wid * kAccWords + k * 32 + lane]; s_acc[wid * kAccWords + k * 32 + lane] = 0; }
-                    finish_chunk<kPpad>(a, un.cell, un.t0 + 32 * wid, lane, cnt, sum, covered, maxd);
+                    finish_chunk_rt<kPpad>(a, un.cell, un.t0 + 32 * wid, lane, cnt, sum, covered, maxd);
                 }
             }
             unit_statistics(a, un.cell, lane, sum, covered, maxd);

@@ -271,6 +271,41 @@ int mgatk_variant_stats_device(mgatk_handle *h, const mgatk_params *params, cons
 int mgatk_variant_cells_device(mgatk_handle *h, const mgatk_params *params, const mgatk_outputs *result_dev,
                                const int32_t *variants_dev, int32_t n_variants, uint32_t *out_dev, void *stream);
 
+/* ---- clones (DESIGN §8, "Clones") -----------------------------------------
+ * Cells grouped into clones by the heteroplasmy of called variants: Signac's AlleleFreq + FindClonotypes, with an
+ * exact kNN search and deterministic Louvain. x[c][v] = (f + r) / d (0 when d = 0) from the counts of
+ * mgatk_variant_cells_device; every float operation is an IEEE fp64 multiply, add, square root or divide (no FMA):
+ *     dot(i, j) = sum over v ascending of acc = acc + x[i][v] * x[j][v], from acc = 0
+ *     inv[i] = 1 / sqrt(dot(i, i)) (0 when dot(i, i) = 0),   cos(i, j) = (dot(i, j) * inv[i]) * inv[j]
+ * N(i) is row i itself with similarity 1.0, then the k_eff - 1 other rows with the largest cos(i, j), ties to the lower
+ * row index (k_eff = min(k, n_rows)). */
+#define MGATK_CLONE_K_MAX 64
+#define MGATK_CLONE_MAX_ROWS (1 << 24)            /* n_rows                                            */
+#define MGATK_CLONE_MAX_VARIANTS 4096             /* n_variants                                        */
+#define MGATK_CLONE_MAX_ELEMENTS ((int64_t)1 << 31) /* n_rows * (n_variants rounded up to 32): x scratch */
+
+/* kNN of the graph rows. counts_dev: uint32 [n_variants][3][n_cells] (alt forward, alt reverse, coverage) as the
+ * variant-cells entry writes it; rows_dev: int32 [n_rows] distinct cell indices in [0, n_cells), each with x > 0 for at
+ * least one variant (the graph rows). A row that breaks this (no detection, or a cell index outside [0, n_cells),
+ * read as zero counts) has cosine 0 with every row, so the result stays defined and deterministic. Writes nbr_out int32 [n_rows][k_eff] (row
+ * indices into rows_dev, N(i) in order) and sim_out fp64 [n_rows][k_eff]. The result does not depend on the launch
+ * configuration. MGATK_ERR_BAD_ARG: k outside [2, MGATK_CLONE_K_MAX], a negative size, a null pointer, n_variants = 0
+ * or n_rows > n_cells with rows; MGATK_ERR_RANGE: beyond the MGATK_CLONE_MAX_* limits. x and inv live in handle
+ * scratch: calls on one handle must be ordered (one stream). */
+int mgatk_clone_knn_device(mgatk_handle *h, const uint32_t *counts_dev, const int32_t *rows_dev, int32_t n_rows,
+                           int32_t n_cells, int32_t n_variants, int32_t k, int32_t *nbr_out, double *sim_out, void *stream);
+/* Shared-nearest-neighbour weight of every directed kNN edge: w_out[i][t] = s / (2 k_eff - s), s = |N(i) ∩ N(j)|,
+ * j = nbr_dev[i][t] (fp64 divide). nbr_dev is [n][k_eff] as the kNN entry writes it. MGATK_ERR_BAD_ARG: negative n,
+ * k_eff outside [1, min(MGATK_CLONE_K_MAX, n)], a null pointer; MGATK_ERR_RANGE: n above MGATK_CLONE_MAX_ROWS. */
+int mgatk_clone_snn_device(mgatk_handle *h, const int32_t *nbr_dev, int32_t n, int32_t k_eff, double *w_out, void *stream);
+/* Deterministic Louvain on the host (no CUDA call, no handle): a symmetric weighted graph in CSR form (indptr int64
+ * [n + 1] from 0, indices int32 ascending within a row, weights fp64 >= 0, diagonal allowed) at `resolution` > 0.
+ * labels_out int32 [n]: clone numbers 1..K by size descending, ties to the smallest member; *n_levels_out: levels whose
+ * first phase moved a node. The rules are those of DESIGN §8 "Clones". MGATK_ERR_BAD_ARG for a malformed graph or
+ * resolution, MGATK_ERR_RANGE for 2^31 or more entries or when memory runs out. */
+int mgatk_louvain_host(int32_t n, const int64_t *indptr, const int32_t *indices, const double *weights, double resolution,
+                       int32_t *labels_out, int32_t *n_levels_out);
+
 /* number of kernel launches issued by the last mgatk_pileup_* call on this handle */
 int64_t mgatk_last_launch_count(const mgatk_handle *h);
 

@@ -14,7 +14,8 @@ __all__ = ["ReadBatch", "PipelineConfig", "QualityThresholds", "DeduplicationCon
            "PileupKernelError", "BAMReader", "CellProcessor", "process_barcode_worker", "PileupGenerator",
            "PileupEngine", "MtDNAPipeline", "run_pipeline", "load_singlecell_csv", "extract_barcodes_from_bam",
            "DenseTextWriter", "DenseHDF5Writer", "report_inputs",
-           "VARIANT_SUMS_DTYPE", "variant_sums", "finalize", "call_variants", "variant_cells"]
+           "VARIANT_SUMS_DTYPE", "variant_sums", "finalize", "call_variants", "variant_cells",
+           "allele_frequencies", "find_clones", "clone_variants"]
 
 
 def __getattr__(name):        # heavy pieces (ctypes library, torch) load on first use
@@ -42,6 +43,9 @@ def __getattr__(name):        # heavy pieces (ctypes library, torch) load on fir
     if name in ("VARIANT_SUMS_DTYPE", "variant_sums", "finalize", "call_variants", "variant_cells"):
         from . import variants
         return getattr(variants, name)
+    if name in ("allele_frequencies", "find_clones", "clone_variants"):
+        from . import clones
+        return getattr(clones, name)
     if name == "PileupEngine":
         from .engine import PileupEngine
         return PileupEngine

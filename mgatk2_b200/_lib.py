@@ -16,6 +16,7 @@ EXPORTS = (
     "mgatk_filter_strand_bias_device", "mgatk_filter_strand_bias_u32_device", "mgatk_stream_begin_device", "mgatk_stream_finish_device",
     "mgatk_last_launch_count", "mgatk_last_stage_times", "mgatk_pileup_host_submit", "mgatk_pileup_host_wait",
     "mgatk_variant_stats_device", "mgatk_variant_cells_device",
+    "mgatk_clone_knn_device", "mgatk_clone_snn_device", "mgatk_louvain_host",
 )
 
 N_PLANES = 11
@@ -98,6 +99,12 @@ def load():
                                                ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p]
     lib.mgatk_variant_cells_device.argtypes = [ctypes.c_void_p, ctypes.POINTER(ParamsC), ctypes.POINTER(OutputsC),
                                                ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p]
+    lib.mgatk_clone_knn_device.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32,
+                                           ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
+    lib.mgatk_clone_snn_device.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p,
+                                           ctypes.c_void_p]
+    lib.mgatk_louvain_host.argtypes = [ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_double,
+                                       ctypes.c_void_p, ctypes.POINTER(ctypes.c_int32)]
     if lib.mgatk_abi_version() != ABI_VERSION:
         raise ExtensionMissingError(f"ABI mismatch: library {lib.mgatk_abi_version()}, binding {ABI_VERSION}")
     _lib = lib

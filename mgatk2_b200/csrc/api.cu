@@ -13,6 +13,7 @@
 #include "pileup.cuh"
 #include "epilogue.cuh"
 #include "variants.cuh"
+#include "clones.cuh"
 
 using namespace mgatk;
 
@@ -132,6 +133,8 @@ struct mgatk_handle {
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     // variant statistics: hash table of the overflow list of the result being reduced
     DevBuf var_table;
+    // clones: x [n][vpad] and inv [n] of the rows being searched
+    DevBuf clone_x;
 };
 
 namespace {
@@ -568,6 +571,7 @@ int mgatk_destroy(mgatk_handle *h) {
     if (h->deep_planes.p) cudaFree(h->deep_planes.p);
     if (h->deep_map.p) cudaFree(h->deep_map.p);
     if (h->var_table.p) cudaFree(h->var_table.p);
+    if (h->clone_x.p) cudaFree(h->clone_x.p);
     if (h->s_h2d) { cudaStreamDestroy(h->s_h2d); cudaStreamDestroy(h->s_d2h); }
     if (h->events_ready) for (int i = 0; i <= kMaxStages; i++) cudaEventDestroy(h->ev[i]);
     if (h->stream) cudaStreamDestroy(h->stream);
@@ -800,6 +804,80 @@ int mgatk_variant_cells_device(mgatk_handle *h, const mgatk_params *p, const mga
     k_variant_cells<<<grid, 256, 0, s>>>(o->planes, table, o->stats, o->overflow_capacity, variants_dev, n_variants, p->n_cells,
                                          p->mito_length, (int)MGATK_POS_PAD(p->mito_length), out_dev);
     CU(cudaGetLastError());
+    return MGATK_OK;
+}
+
+int mgatk_clone_knn_device(mgatk_handle *h, const uint32_t *counts_dev, const int32_t *rows_dev, int32_t n_rows,
+                           int32_t n_cells, int32_t n_variants, int32_t k, int32_t *nbr_out, double *sim_out, void *stream) {
+    if (!h) return MGATK_ERR_BAD_ARG;
+    h->err.clear();
+    if (k < 2 || k > MGATK_CLONE_K_MAX) return fail(h, MGATK_ERR_BAD_ARG, "k must be in [2, 64]");
+    if (n_rows < 0 || n_cells < 0 || n_variants < 0) return fail(h, MGATK_ERR_BAD_ARG, "negative size");
+    if (n_rows == 0) return MGATK_OK;
+    if (!rows_dev || !nbr_out || !sim_out || !counts_dev) return fail(h, MGATK_ERR_BAD_ARG, "null argument");
+    if (n_variants == 0 || n_rows > n_cells) return fail(h, MGATK_ERR_BAD_ARG, "graph rows need a variant and distinct cells");
+    if (n_rows > MGATK_CLONE_MAX_ROWS || n_variants > MGATK_CLONE_MAX_VARIANTS)
+        return fail(h, MGATK_ERR_RANGE, "n_rows above 2^24 or n_variants above 4096");
+    const int vpad = clone_vpad(n_variants);
+    if ((int64_t)n_rows * vpad > MGATK_CLONE_MAX_ELEMENTS) return fail(h, MGATK_ERR_RANGE, "n_rows * padded n_variants above 2^31");
+    CU(cudaSetDevice(h->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    const int k_eff = k < n_rows ? k : n_rows;
+    if (k_eff == 1) {
+        k_clone_self<<<1, 32, 0, s>>>(n_rows, k_eff, nbr_out, sim_out);
+        CU(cudaGetLastError());
+        return MGATK_OK;
+    }
+    int rc = ensure(h, h->clone_x, ((size_t)n_rows * vpad + n_rows) * sizeof(double));
+    if (rc) return rc;
+    double *x = (double *)h->clone_x.p, *inv = x + (size_t)n_rows * vpad;
+    k_clone_af<<<(unsigned)((n_rows + 127) / 128), 128, 0, s>>>(counts_dev, rows_dev, n_rows, n_cells, n_variants, vpad, x, inv);
+    CU(cudaGetLastError());
+    const int smem = (int)sizeof(CloneKnnSmem);
+    CU(cudaFuncSetAttribute(k_clone_knn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    k_clone_knn<<<(unsigned)((n_rows + kCloneTile - 1) / kCloneTile), kCloneThreads, smem, s>>>(x, inv, n_rows, vpad, k_eff,
+                                                                                                nbr_out, sim_out);
+    CU(cudaGetLastError());
+    return MGATK_OK;
+}
+
+int mgatk_clone_snn_device(mgatk_handle *h, const int32_t *nbr_dev, int32_t n, int32_t k_eff, double *w_out, void *stream) {
+    if (!h) return MGATK_ERR_BAD_ARG;
+    h->err.clear();
+    if (n < 0) return fail(h, MGATK_ERR_BAD_ARG, "negative size");
+    if (n == 0) return MGATK_OK;
+    if (k_eff < 1 || k_eff > MGATK_CLONE_K_MAX || k_eff > n) return fail(h, MGATK_ERR_BAD_ARG, "k_eff must be in [1, min(64, n)]");
+    if (!nbr_dev || !w_out) return fail(h, MGATK_ERR_BAD_ARG, "null argument");
+    if (n > MGATK_CLONE_MAX_ROWS) return fail(h, MGATK_ERR_RANGE, "n above 2^24");
+    CU(cudaSetDevice(h->device));
+    k_clone_snn<<<(unsigned)((n + kSnnWarps - 1) / kSnnWarps), kSnnWarps * 32, 0, (cudaStream_t)stream>>>(nbr_dev, n, k_eff, w_out);
+    CU(cudaGetLastError());
+    return MGATK_OK;
+}
+
+int mgatk_louvain_host(int32_t n, const int64_t *indptr, const int32_t *indices, const double *weights, double resolution,
+                       int32_t *labels_out, int32_t *n_levels_out) {
+    if (n < 0 || !n_levels_out || !(resolution > 0.0) || !std::isfinite(resolution)) return MGATK_ERR_BAD_ARG;
+    *n_levels_out = 0;
+    if (n == 0) return MGATK_OK;
+    if (!indptr || !labels_out) return MGATK_ERR_BAD_ARG;
+    if (indptr[0] != 0) return MGATK_ERR_BAD_ARG;
+    for (int32_t i = 0; i < n; i++)
+        if (indptr[i + 1] < indptr[i]) return MGATK_ERR_BAD_ARG;
+    const int64_t nnz = indptr[n];
+    if (nnz > 0 && (!indices || !weights)) return MGATK_ERR_BAD_ARG;
+    if (nnz >= ((int64_t)1 << 31)) return MGATK_ERR_RANGE;
+    for (int64_t e = 0; e < nnz; e++)
+        if (indices[e] < 0 || indices[e] >= n || !(weights[e] >= 0.0) || !std::isfinite(weights[e])) return MGATK_ERR_BAD_ARG;
+    try {
+        LouvainGraph g;
+        g.indptr.assign(indptr, indptr + n + 1);
+        g.indices.assign(indices, indices + nnz);
+        g.weights.assign(weights, weights + nnz);
+        louvain(std::move(g), resolution, labels_out, n_levels_out);
+    } catch (const std::bad_alloc &) {
+        return MGATK_ERR_RANGE;
+    }
     return MGATK_OK;
 }
 

@@ -39,9 +39,10 @@ class MtDNAPipeline:
                  output_format: str = "standard", barcode_metadata=None, sample_name: str = "mgatk2",
                  report_title: str | None = None, report_subtitle: str | None = None, working_directory: str | None = None,
                  device: int = 0, devices: list | None = None, max_batch_records: int | None = None,
-                 call_variants: bool = False):
+                 call_variants: bool = False, find_clones: bool = False):
         """`call_variants=True` adds `output/variant_stats.tsv.gz` and `output/variant_cells.tsv.gz` (variants.py) after
-        the reference's outputs, which stay as they are."""
+        the reference's outputs, which stay as they are. `find_clones=True` implies it and adds `output/clones.tsv.gz` and
+        `output/clone_variants.tsv.gz` (clones.py, the called variants, default parameters)."""
         self.bam_path = Path(bam_path)
         self.barcodes = set(barcodes)
         self.barcode_list = list(barcodes)
@@ -53,7 +54,8 @@ class MtDNAPipeline:
         self.devices = list(devices) if devices else [device]      # GPUs of this box; the cells are split between them
         self.device = self.devices[0]
         self.max_batch_records = max_batch_records                  # larger contigs are streamed in parts (dispatch.py)
-        self.call_variants = bool(call_variants)
+        self.find_clones = bool(find_clones)
+        self.call_variants = bool(call_variants) or self.find_clones
         if not self.bam_path.exists():
             raise InvalidInputError(f"BAM file not found: {bam_path}")
         from .bamio import BamFile, pick_mito_contig
@@ -93,10 +95,14 @@ class MtDNAPipeline:
         writer.finalize(qc_dir)
         if self.call_variants:
             from .pileup import get_engine
-            from .variants import write_variant_files
-            called = write_variant_files(reads_by_barcode.result, self.barcode_list, self.output_dir / "output",
-                                         engine=get_engine(self.device))
+            from .variants import _Source, write_variant_files
+            src = _Source(reads_by_barcode.result, get_engine(self.device))         # one upload for every file below
+            called, counts = write_variant_files(src, self.barcode_list, self.output_dir / "output")
             logger.info("%d variants called", len(called))
+            if self.find_clones:
+                from .clones import write_clone_files
+                clones = write_clone_files(src, self.barcode_list, self.output_dir / "output", called, counts)
+                logger.info("%d clones", clones.n_clones)
         self.timings = dict(getattr(reader, "timings", {}), write_s=time.time() - t_write, total_s=time.time() - start)
         c = self.config
         write_run_summary({                                               # analysis/qc.py:68-93
@@ -119,13 +125,14 @@ class MtDNAPipeline:
 def run_pipeline(bam_path: str, output_dir: str, barcode_file: str | None = None, min_barcode_reads: int = 10,
                  barcode_tag: str = "CB", mito_chr: str = "chrM", output_format: str = "standard", device: int = 0,
                  devices: list | None = None, max_batch_records: int | None = None, call_variants: bool = False,
-                 **config_kwargs) -> dict:
+                 find_clones: bool = False, **config_kwargs) -> dict:
     """core.pipeline.run_pipeline (pipeline.py:184-270): whitelist from file / singlecell.csv / the BAM itself, then
-    `MtDNAPipeline.run()` (`call_variants`: as there). `config_kwargs` are `PipelineConfig` keywords (min_baseq, min_mapq, max_strand_bias,
+    `MtDNAPipeline.run()` (`call_variants`, `find_clones`: as there). `config_kwargs` are `PipelineConfig` keywords (min_baseq, min_mapq, max_strand_bias,
     skip_deduplication, use_fragment_length_dedup, min_reads_per_cell, ...)."""
     barcodes, metadata = load_barcodes(barcode_file, bam_path, barcode_tag=barcode_tag, mito_chr=mito_chr,
                                        min_barcode_reads=min_barcode_reads)
     config = PipelineConfig(barcode_tag=barcode_tag, mito_chr=mito_chr, **config_kwargs)
     return MtDNAPipeline(bam_path, barcodes, Path(output_dir), config, output_format=output_format,
                          barcode_metadata=metadata, device=device, devices=devices,
-                         max_batch_records=max_batch_records, call_variants=call_variants).run()
+                         max_batch_records=max_batch_records, call_variants=call_variants,
+                         find_clones=find_clones).run()

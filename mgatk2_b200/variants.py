@@ -146,6 +146,7 @@ class _Source:
                                     ov.data_ptr() if len(ovf) else None, len(ovf))
             self.params = _params(C, P)
             self.qc, self.min_reads = res.cell_qc, res.min_reads_per_cell
+            self.columns = None if res.columns is None else np.asarray(res.columns)
         else:
             dout, params = source
             self.engine = engine or get_engine(dout.planes.device.index)
@@ -161,11 +162,17 @@ class _Source:
             self.params = _params(C, P)
             self.qc = dout.cell_qc.cpu().numpy().view(CELL_QC_DTYPE)[:C]
             self.min_reads = int(params.min_reads_per_cell)
+            self.columns = None
         self.n_cells, self.mito_length = C, P
 
     def alive(self) -> np.ndarray:
         n = self.qc["n_reads"].astype(np.int64)
         return (n >= max(1, self.min_reads)) & (self.qc["sum_depth"] > 0)
+
+    def barcodes(self, barcode_list) -> list:
+        """The name of every row: barcode_list[columns[k]] (row k is whitelist entry k without columns)."""
+        rows = range(self.n_cells) if self.columns is None else self.columns.tolist()
+        return [barcode_list[int(c)] for c in rows]
 
     def stream(self):
         import torch
@@ -228,9 +235,9 @@ def variant_ids(variants) -> np.ndarray:
     return v.astype(np.int32).reshape(-1)
 
 
-def variant_cells(source, variants, engine=None) -> np.ndarray:
-    """uint32 [n_variants, 3, n_cells]: exact alt forward, alt reverse and coverage of every row of `source` for every
-    variant (mgatk_variant_cells_device). `variants` is a table of finalize or int ids pos * 4 + alt."""
+def variant_cells_device(source, variants, engine=None):
+    """The counts of variant_cells left on the GPU: a torch int32 tensor [n_variants, 3, n_cells] holding the uint32
+    values (enqueued on the current stream)."""
     import torch
     src = source if isinstance(source, _Source) else _Source(source, engine)
     ids = variant_ids(variants)
@@ -244,7 +251,14 @@ def variant_cells(source, variants, engine=None) -> np.ndarray:
                                                    ids_t.data_ptr(), n, out.data_ptr(), src.stream())
     if rc:
         src.engine._raise(rc)
-    return out.cpu().numpy().view(np.uint32)[: n * 3 * src.n_cells].reshape(n, 3, src.n_cells).copy()
+    return out[: n * 3 * src.n_cells].view(n, 3, src.n_cells)
+
+
+def variant_cells(source, variants, engine=None) -> np.ndarray:
+    """uint32 [n_variants, 3, n_cells]: exact alt forward, alt reverse and coverage of every row of `source` for every
+    variant (mgatk_variant_cells_device). `variants` is a table of finalize or int ids pos * 4 + alt."""
+    out = variant_cells_device(source, variants, engine)
+    return out.cpu().numpy().view(np.uint32).copy()
 
 
 # ---------------------------------------------------------------------------------------------------------------- files
@@ -289,18 +303,17 @@ def read_variant_stats(path) -> np.ndarray:
     return t
 
 
-def write_variant_files(result: PileupResult, barcode_list, output_dir, engine=None, low_coverage_threshold: int = 10,
-                        **call_kwargs) -> np.ndarray:
+def write_variant_files(result, barcode_list, output_dir, engine=None, low_coverage_threshold: int = 10, **call_kwargs):
     """`output_dir/variant_stats.tsv.gz` and `output_dir/variant_cells.tsv.gz` for the cells with a QC row of a host
-    result; barcodes are `barcode_list[columns[k]]` for row k. Returns the called variants."""
-    src = _Source(result, engine)                      # planes uploaded once for both calls
+    result (or a `_Source` of one, so later steps reuse its upload); barcodes are `barcode_list[columns[k]]` for row k.
+    Returns the called variants and their counts (variant_cells)."""
+    src = result if isinstance(result, _Source) else _Source(result, engine)     # planes uploaded once for both calls
     mask = src.alive()
     sums = variant_sums(src, cells=mask, low_coverage_threshold=low_coverage_threshold)
     table = finalize(sums, int(mask.sum()))
     called = call_variants(table, **call_kwargs)
-    rows = np.arange(len(result.planes)) if result.columns is None else np.asarray(result.columns)
-    names = [barcode_list[int(c)] for c in rows.tolist()]
+    counts = variant_cells(src, called)
     out = Path(output_dir)
     write_variant_stats(table, out / "variant_stats.tsv.gz")
-    write_variant_cells(called, variant_cells(src, called), names, mask, out / "variant_cells.tsv.gz")
-    return called
+    write_variant_cells(called, counts, src.barcodes(barcode_list), mask, out / "variant_cells.tsv.gz")
+    return called, counts

@@ -306,6 +306,25 @@ int mgatk_clone_snn_device(mgatk_handle *h, const int32_t *nbr_dev, int32_t n, i
 int mgatk_louvain_host(int32_t n, const int64_t *indptr, const int32_t *indices, const double *weights, double resolution,
                        int32_t *labels_out, int32_t *n_levels_out);
 
+/* ---- clone markers (DESIGN §8, "Clone markers") ------------------------------
+ * Seurat's FindAllMarkers test on the heteroplasmy of variants: a two-sided Wilcoxon rank-sum test per variant, each
+ * group of cells against the other cells of the population. x = (f + r) / d as for the clones (0 when d = 0); the
+ * population is the cells with a label in [1, n_groups], N their number; rank(c) is the 1-based mid-rank of x[v][c]
+ * among the population. The device gives exact integers; the host forms U, the tie-corrected normal approximation and
+ * p from them. */
+#define MGATK_MARKER_MAX_CELLS (1 << 21)          /* n_cells: N^3 stays below 2^63                       */
+
+/* Wilcoxon rank sums of x = (f + r) / d per variant: counts_dev uint32 [n_variants][3][n_cells] as
+ * mgatk_variant_cells_device writes it, labels_dev int32 [n_cells] (1..n_groups: a group; anything else: not in
+ * the test). rank2_out uint64 [n_variants][n_groups] = sum over the group's cells of 2 * mid-rank, ties_out uint64
+ * [n_variants] = sum over runs of equal x of t^3 - t. Every output entry is written; integer results, so they do not
+ * depend on the launch configuration. Scratch lives in the handle (calls on one handle ordered, freed by
+ * mgatk_destroy). MGATK_ERR_BAD_ARG: a null pointer with a non-zero size, a negative size, n_groups < 1;
+ * MGATK_ERR_RANGE: n_cells above MGATK_MARKER_MAX_CELLS, n_variants above MGATK_CLONE_MAX_VARIANTS, n_groups above
+ * n_cells (n_cells > 0). n_variants = 0 or n_cells = 0: MGATK_OK (outputs zero when n_cells = 0). */
+int mgatk_marker_ranks_device(mgatk_handle *h, const uint32_t *counts_dev, const int32_t *labels_dev, int32_t n_cells,
+                              int32_t n_variants, int32_t n_groups, uint64_t *rank2_out, uint64_t *ties_out, void *stream);
+
 /* number of kernel launches issued by the last mgatk_pileup_* call on this handle */
 int64_t mgatk_last_launch_count(const mgatk_handle *h);
 

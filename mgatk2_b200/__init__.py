@@ -15,7 +15,7 @@ __all__ = ["ReadBatch", "PipelineConfig", "QualityThresholds", "DeduplicationCon
            "PileupEngine", "MtDNAPipeline", "run_pipeline", "load_singlecell_csv", "extract_barcodes_from_bam",
            "DenseTextWriter", "DenseHDF5Writer", "report_inputs",
            "VARIANT_SUMS_DTYPE", "variant_sums", "finalize", "call_variants", "variant_cells",
-           "allele_frequencies", "find_clones", "clone_variants"]
+           "allele_frequencies", "find_clones", "clone_variants", "find_markers", "clone_markers"]
 
 
 def __getattr__(name):        # heavy pieces (ctypes library, torch) load on first use
@@ -46,6 +46,9 @@ def __getattr__(name):        # heavy pieces (ctypes library, torch) load on fir
     if name in ("allele_frequencies", "find_clones", "clone_variants"):
         from . import clones
         return getattr(clones, name)
+    if name in ("find_markers", "clone_markers"):
+        from . import markers
+        return getattr(markers, name)
     if name == "PileupEngine":
         from .engine import PileupEngine
         return PileupEngine

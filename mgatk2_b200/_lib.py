@@ -16,7 +16,7 @@ EXPORTS = (
     "mgatk_filter_strand_bias_device", "mgatk_filter_strand_bias_u32_device", "mgatk_stream_begin_device", "mgatk_stream_finish_device",
     "mgatk_last_launch_count", "mgatk_last_stage_times", "mgatk_pileup_host_submit", "mgatk_pileup_host_wait",
     "mgatk_variant_stats_device", "mgatk_variant_cells_device",
-    "mgatk_clone_knn_device", "mgatk_clone_snn_device", "mgatk_louvain_host",
+    "mgatk_clone_knn_device", "mgatk_clone_snn_device", "mgatk_louvain_host", "mgatk_marker_ranks_device",
 )
 
 N_PLANES = 11
@@ -105,6 +105,9 @@ def load():
                                            ctypes.c_void_p]
     lib.mgatk_louvain_host.argtypes = [ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_double,
                                        ctypes.c_void_p, ctypes.POINTER(ctypes.c_int32)]
+    lib.mgatk_marker_ranks_device.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32,
+                                              ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p,
+                                              ctypes.c_void_p]
     if lib.mgatk_abi_version() != ABI_VERSION:
         raise ExtensionMissingError(f"ABI mismatch: library {lib.mgatk_abi_version()}, binding {ABI_VERSION}")
     _lib = lib

@@ -14,6 +14,7 @@
 #include "epilogue.cuh"
 #include "variants.cuh"
 #include "clones.cuh"
+#include "markers.cuh"
 
 using namespace mgatk;
 
@@ -135,6 +136,8 @@ struct mgatk_handle {
     DevBuf var_table;
     // clones: x [n][vpad] and inv [n] of the rows being searched
     DevBuf clone_x;
+    // clone markers: the nonzero (x, label) pairs of every variant, the fallback's ping-pong pairs, the counters
+    DevBuf marker_scratch;
 };
 
 namespace {
@@ -572,6 +575,7 @@ int mgatk_destroy(mgatk_handle *h) {
     if (h->deep_map.p) cudaFree(h->deep_map.p);
     if (h->var_table.p) cudaFree(h->var_table.p);
     if (h->clone_x.p) cudaFree(h->clone_x.p);
+    if (h->marker_scratch.p) cudaFree(h->marker_scratch.p);
     if (h->s_h2d) { cudaStreamDestroy(h->s_h2d); cudaStreamDestroy(h->s_d2h); }
     if (h->events_ready) for (int i = 0; i <= kMaxStages; i++) cudaEventDestroy(h->ev[i]);
     if (h->stream) cudaStreamDestroy(h->stream);
@@ -851,6 +855,49 @@ int mgatk_clone_snn_device(mgatk_handle *h, const int32_t *nbr_dev, int32_t n, i
     if (n > MGATK_CLONE_MAX_ROWS) return fail(h, MGATK_ERR_RANGE, "n above 2^24");
     CU(cudaSetDevice(h->device));
     k_clone_snn<<<(unsigned)((n + kSnnWarps - 1) / kSnnWarps), kSnnWarps * 32, 0, (cudaStream_t)stream>>>(nbr_dev, n, k_eff, w_out);
+    CU(cudaGetLastError());
+    return MGATK_OK;
+}
+
+int mgatk_marker_ranks_device(mgatk_handle *h, const uint32_t *counts_dev, const int32_t *labels_dev, int32_t n_cells,
+                              int32_t n_variants, int32_t n_groups, uint64_t *rank2_out, uint64_t *ties_out, void *stream) {
+    if (!h) return MGATK_ERR_BAD_ARG;
+    h->err.clear();
+    if (n_cells < 0 || n_variants < 0) return fail(h, MGATK_ERR_BAD_ARG, "negative size");
+    if (n_groups < 1) return fail(h, MGATK_ERR_BAD_ARG, "n_groups must be >= 1");
+    if ((n_cells > 0 && !labels_dev) || (n_cells > 0 && n_variants > 0 && !counts_dev) ||
+        (n_variants > 0 && (!rank2_out || !ties_out)))
+        return fail(h, MGATK_ERR_BAD_ARG, "null argument");
+    if (n_cells > MGATK_MARKER_MAX_CELLS || n_variants > MGATK_CLONE_MAX_VARIANTS)
+        return fail(h, MGATK_ERR_RANGE, "n_cells above 2^21 or n_variants above 4096");
+    if (n_cells > 0 && n_groups > n_cells) return fail(h, MGATK_ERR_RANGE, "n_groups above n_cells");
+    if (n_variants == 0) return MGATK_OK;
+    CU(cudaSetDevice(h->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t V = (size_t)n_variants, C = (size_t)n_cells, G = (size_t)n_groups;
+    if (n_cells == 0) {
+        CU(cudaMemsetAsync(rank2_out, 0, V * G * sizeof(uint64_t), s));
+        CU(cudaMemsetAsync(ties_out, 0, V * sizeof(uint64_t), s));
+        return MGATK_OK;
+    }
+    const int grid = n_variants < 2 * h->sm_count ? n_variants : 2 * h->sm_count;
+    const size_t tmp = n_cells > kMarkerS ? (size_t)grid * C : 0;       // the fallback needs ping-pong pairs
+    const size_t o_tkeys = align_up(V * C * 8), o_labs = o_tkeys + align_up(tmp * 8), o_tlabs = o_labs + align_up(V * C * 4);
+    const size_t o_cnt = o_tlabs + align_up(tmp * 4), n_cnt = V + G + 2;
+    int rc = ensure(h, h->marker_scratch, o_cnt + n_cnt * 4);
+    if (rc) return rc;
+    char *base = (char *)h->marker_scratch.p;
+    u32 *nnz = (u32 *)(base + o_cnt), *gsize = nnz + V, *npop = gsize + G + 1;
+    CU(cudaMemsetAsync(nnz, 0, n_cnt * 4, s));
+    dim3 sg((unsigned)((C + kMarkerSplitThreads - 1) / kMarkerSplitThreads), (unsigned)V);
+    k_marker_split<<<sg, kMarkerSplitThreads, 0, s>>>(counts_dev, labels_dev, n_cells, n_groups, nnz, gsize, npop,
+                                                      (u64 *)base, (int32_t *)(base + o_labs));
+    CU(cudaGetLastError());
+    const int smem = (int)sizeof(MarkerSmem);
+    CU(cudaFuncSetAttribute(k_marker_rank, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    k_marker_rank<<<grid, kMarkerThreads, smem, s>>>((u64 *)base, (int32_t *)(base + o_labs), nnz, gsize, npop, n_cells,
+                                                     n_variants, n_groups, (u64 *)(base + o_tkeys),
+                                                     (int32_t *)(base + o_tlabs), (u64 *)rank2_out, (u64 *)ties_out);
     CU(cudaGetLastError());
     return MGATK_OK;
 }

@@ -31,6 +31,14 @@ constexpr int kClonePitch = kCloneTile + 1;
 
 __host__ __device__ inline int clone_vpad(int V) { return (V + kCloneVC - 1) / kCloneVC * kCloneVC; }
 
+// x = (f + r) / d of cell c in variant v, 0 when d = 0; counts is [V][3][C] of mgatk_variant_cells_device (also the x of
+// the marker ranks, markers.cuh)
+__device__ __forceinline__ double allele_frequency(const u32 *counts, int C, int v, int c) {
+    const u32 *cv = counts + (size_t)3 * v * C + c;
+    const u32 d = cv[2 * (size_t)C];
+    return d ? __ddiv_rn((double)((u64)cv[0] + cv[C]), (double)d) : 0.0;
+}
+
 // x[i][v] and inv[i] of graph row i (cell rows[i]); counts is [V][3][C] of mgatk_variant_cells_device
 __global__ void k_clone_af(const u32 *counts, const int32_t *rows, int n, int C, int V, int vpad, double *x, double *inv) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -39,12 +47,7 @@ __global__ void k_clone_af(const u32 *counts, const int32_t *rows, int n, int C,
     const bool ok = c >= 0 && c < C;
     double acc = 0.0;
     for (int v = 0; v < vpad; v++) {
-        double xv = 0.0;
-        if (ok && v < V) {
-            const u32 *cv = counts + (size_t)3 * v * C + c;
-            const u32 d = cv[2 * (size_t)C];
-            if (d) xv = __ddiv_rn((double)((u64)cv[0] + cv[C]), (double)d);
-        }
+        const double xv = ok && v < V ? allele_frequency(counts, C, v, c) : 0.0;
         x[(size_t)i * vpad + v] = xv;
         acc = __dadd_rn(acc, __dmul_rn(xv, xv));
     }

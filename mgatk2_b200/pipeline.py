@@ -39,10 +39,11 @@ class MtDNAPipeline:
                  output_format: str = "standard", barcode_metadata=None, sample_name: str = "mgatk2",
                  report_title: str | None = None, report_subtitle: str | None = None, working_directory: str | None = None,
                  device: int = 0, devices: list | None = None, max_batch_records: int | None = None,
-                 call_variants: bool = False, find_clones: bool = False):
+                 call_variants: bool = False, find_clones: bool = False, clone_markers: bool = False):
         """`call_variants=True` adds `output/variant_stats.tsv.gz` and `output/variant_cells.tsv.gz` (variants.py) after
         the reference's outputs, which stay as they are. `find_clones=True` implies it and adds `output/clones.tsv.gz` and
-        `output/clone_variants.tsv.gz` (clones.py, the called variants, default parameters)."""
+        `output/clone_variants.tsv.gz` (clones.py, the called variants, default parameters). `clone_markers=True` implies
+        `find_clones` and adds `output/clone_markers.tsv.gz` (markers.py: each clone against the other graph cells)."""
         self.bam_path = Path(bam_path)
         self.barcodes = set(barcodes)
         self.barcode_list = list(barcodes)
@@ -54,7 +55,8 @@ class MtDNAPipeline:
         self.devices = list(devices) if devices else [device]      # GPUs of this box; the cells are split between them
         self.device = self.devices[0]
         self.max_batch_records = max_batch_records                  # larger contigs are streamed in parts (dispatch.py)
-        self.find_clones = bool(find_clones)
+        self.clone_markers = bool(clone_markers)
+        self.find_clones = bool(find_clones) or self.clone_markers
         self.call_variants = bool(call_variants) or self.find_clones
         if not self.bam_path.exists():
             raise InvalidInputError(f"BAM file not found: {bam_path}")
@@ -103,6 +105,10 @@ class MtDNAPipeline:
                 from .clones import write_clone_files
                 clones = write_clone_files(src, self.barcode_list, self.output_dir / "output", called, counts)
                 logger.info("%d clones", clones.n_clones)
+                if self.clone_markers:
+                    from .markers import clone_markers, write_clone_markers
+                    write_clone_markers(clone_markers(src, clones, counts=counts),
+                                        self.output_dir / "output" / "clone_markers.tsv.gz")
         self.timings = dict(getattr(reader, "timings", {}), write_s=time.time() - t_write, total_s=time.time() - start)
         c = self.config
         write_run_summary({                                               # analysis/qc.py:68-93
@@ -125,9 +131,9 @@ class MtDNAPipeline:
 def run_pipeline(bam_path: str, output_dir: str, barcode_file: str | None = None, min_barcode_reads: int = 10,
                  barcode_tag: str = "CB", mito_chr: str = "chrM", output_format: str = "standard", device: int = 0,
                  devices: list | None = None, max_batch_records: int | None = None, call_variants: bool = False,
-                 find_clones: bool = False, **config_kwargs) -> dict:
+                 find_clones: bool = False, clone_markers: bool = False, **config_kwargs) -> dict:
     """core.pipeline.run_pipeline (pipeline.py:184-270): whitelist from file / singlecell.csv / the BAM itself, then
-    `MtDNAPipeline.run()` (`call_variants`, `find_clones`: as there). `config_kwargs` are `PipelineConfig` keywords (min_baseq, min_mapq, max_strand_bias,
+    `MtDNAPipeline.run()` (`call_variants`, `find_clones`, `clone_markers`: as there). `config_kwargs` are `PipelineConfig` keywords (min_baseq, min_mapq, max_strand_bias,
     skip_deduplication, use_fragment_length_dedup, min_reads_per_cell, ...)."""
     barcodes, metadata = load_barcodes(barcode_file, bam_path, barcode_tag=barcode_tag, mito_chr=mito_chr,
                                        min_barcode_reads=min_barcode_reads)
@@ -135,4 +141,4 @@ def run_pipeline(bam_path: str, output_dir: str, barcode_file: str | None = None
     return MtDNAPipeline(bam_path, barcodes, Path(output_dir), config, output_format=output_format,
                          barcode_metadata=metadata, device=device, devices=devices,
                          max_batch_records=max_batch_records, call_variants=call_variants,
-                         find_clones=find_clones).run()
+                         find_clones=find_clones, clone_markers=clone_markers).run()

@@ -152,7 +152,8 @@ typedef struct mgatk_stats {
     uint64_t dup_position_only;/* stats["duplicate_reads_position_only"]                */
     uint64_t n_empty_seq;      /* dedup survivors with l_seq==0 (reference raises)      */
     uint64_t n_overflow;       /* entries written to the overflow list                  */
-    uint64_t error_bits;       /* bit0 unsorted, bit1 extent, bit2 overflow capacity, bit3 stream saturated */
+    uint64_t error_bits;       /* bit0 unsorted, bit1 extent, bit2 overflow capacity, bit3 stream saturated,
+                                  bit4 a deletion out of range (mgatk_deletion_scan_device) */
 } mgatk_stats;
 
 /* exact value of one saturated plane entry */
@@ -324,6 +325,46 @@ int mgatk_louvain_host(int32_t n, const int64_t *indptr, const int32_t *indices,
  * n_cells (n_cells > 0). n_variants = 0 or n_cells = 0: MGATK_OK (outputs zero when n_cells = 0). */
 int mgatk_marker_ranks_device(mgatk_handle *h, const uint32_t *counts_dev, const int32_t *labels_dev, int32_t n_cells,
                               int32_t n_variants, int32_t n_groups, uint64_t *rank2_out, uint64_t *ties_out, void *stream);
+
+/* ---- deletions (DESIGN §8, "Deletions") ---------------------------------------
+ * Large mtDNA deletions from the reads themselves, as mgatk-del does: soft-clip breakpoints and, per cell, the reads that
+ * show a junction against the reads that span a breakpoint. The reads are those the pileup counts: stage 1
+ * (flag & 0x904 == 0, 0 <= bc_idx < n_cells), dedup per params->dedup_mode and barcode with the first record of a key in
+ * file order surviving, then mapq >= min_mapq (after dedup). Per read: a0 = pos, a1 = pos + span - 1 (span = sum of
+ * M/D/N/=/X; span 0 takes no part), sl / sr = the S ops before the first / after the last M/=/X op (0 when longer than
+ * SEQ or without such an op). A deletion is (l, r): l the last kept position before the deleted segment, r the first one
+ * after it, 0 <= l, l + 1 < r < P (HGVS m.{l+2}_{r}del). Per read and deletion, at most one class:
+ *     clip_left   a1 = l and sr >= min_clip          clip_right   a0 = r and sl >= min_clip
+ *     gap         a D or N op over exactly [l + 1, r)
+ *     wt          one M/=/X block covers l and l + 1, or r - 1 and r
+ * Discovery histograms over all reads and cells: end_clip[p] reads with sr >= min_clip and a1 = p; start_clip[p] reads
+ * with sl >= min_clip and a0 = p; end_seq[p][j][b] / start_seq[p][j][b] the base b (A, C, G, T; other codes are not
+ * counted) of those reads at SEQ[l_seq - sr + j] / SEQ[sl - 1 - j], j < min(MGATK_DEL_KMER, clip). */
+#define MGATK_DEL_KMER 16
+#define MGATK_DEL_MAX 1024                        /* n_deletions */
+
+/* One part of a coordinate-sorted input (parts cut on reference_start borders add up: dedup keys only repeat within a
+ * run of equal starts). left_dev / right_dev: int32 [n_deletions] device arrays of l and r. Every output is ADDED to, so
+ * the caller zeroes them once and calls once per part:
+ *     counts_out     uint32 [n_deletions][4][n_cells]: clip_left, clip_right, gap, wt
+ *     clip_hist_out  uint64 [2][P]: end_clip, start_clip; NULL = no discovery
+ *     clip_seq_out   uint64 [2][P][MGATK_DEL_KMER][4]: end_seq, start_seq; NULL exactly when clip_hist_out is
+ *     error_bits_out uint64 [1], OR-ed with the bits of mgatk_stats.error_bits: 1 records not sorted by reference_start,
+ *                    2 a stage-1 read longer than params->max_read_extent (l_seq of every one, the reference span of every
+ *                    one whose CIGAR is read: those near a breakpoint, or all with discovery), 16 a deletion outside
+ *                    0 <= l, l + 1 < r < P (it matches nothing). mgatk_check_stats maps them to MGATK_ERR_UNSORTED,
+ *                    MGATK_ERR_EXTENT and MGATK_ERR_RANGE once the stream has drained.
+ * params supplies min_mapq, dedup_mode, n_cells, mito_length (P) and max_read_extent. Integer results: they do not depend
+ * on the launch configuration. Enqueues on `stream`; scratch (about 36 bytes per record) lives in the handle, so calls on
+ * one handle must be ordered; mgatk_destroy frees it. MGATK_ERR_BAD_ARG: a null pointer where data is needed, a negative
+ * size, min_clip < 1, dedup_mode outside 0..2, max_read_extent < 1, a blob not 16-byte aligned, only one of clip_hist_out
+ * and clip_seq_out; MGATK_ERR_EXTENT: max_read_extent above 2^20; MGATK_ERR_RANGE: n_deletions above MGATK_DEL_MAX,
+ * mito_length of 2^24 or more, 2^31 - 256 records or more. No records, or no deletions without discovery: MGATK_OK and
+ * nothing is enqueued. */
+int mgatk_deletion_scan_device(mgatk_handle *h, const mgatk_params *params, const mgatk_batch *batch_dev,
+                               int32_t min_clip, const int32_t *left_dev, const int32_t *right_dev, int32_t n_deletions,
+                               uint32_t *counts_out, uint64_t *clip_hist_out, uint64_t *clip_seq_out,
+                               uint64_t *error_bits_out, void *stream);
 
 /* number of kernel launches issued by the last mgatk_pileup_* call on this handle */
 int64_t mgatk_last_launch_count(const mgatk_handle *h);

@@ -15,7 +15,8 @@ __all__ = ["ReadBatch", "PipelineConfig", "QualityThresholds", "DeduplicationCon
            "PileupEngine", "MtDNAPipeline", "run_pipeline", "load_singlecell_csv", "extract_barcodes_from_bam",
            "DenseTextWriter", "DenseHDF5Writer", "report_inputs",
            "VARIANT_SUMS_DTYPE", "variant_sums", "finalize", "call_variants", "variant_cells",
-           "allele_frequencies", "find_clones", "clone_variants", "find_markers", "clone_markers"]
+           "allele_frequencies", "find_clones", "clone_variants", "find_markers", "clone_markers",
+           "scan_deletions", "find_deletions", "deletion_heteroplasmy"]
 
 
 def __getattr__(name):        # heavy pieces (ctypes library, torch) load on first use
@@ -49,6 +50,9 @@ def __getattr__(name):        # heavy pieces (ctypes library, torch) load on fir
     if name in ("find_markers", "clone_markers"):
         from . import markers
         return getattr(markers, name)
+    if name in ("scan_deletions", "find_deletions", "deletion_heteroplasmy"):
+        from . import deletions
+        return getattr(deletions, name)
     if name == "PileupEngine":
         from .engine import PileupEngine
         return PileupEngine

@@ -17,6 +17,7 @@ EXPORTS = (
     "mgatk_last_launch_count", "mgatk_last_stage_times", "mgatk_pileup_host_submit", "mgatk_pileup_host_wait",
     "mgatk_variant_stats_device", "mgatk_variant_cells_device",
     "mgatk_clone_knn_device", "mgatk_clone_snn_device", "mgatk_louvain_host", "mgatk_marker_ranks_device",
+    "mgatk_deletion_scan_device",
 )
 
 N_PLANES = 11
@@ -108,6 +109,10 @@ def load():
     lib.mgatk_marker_ranks_device.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32,
                                               ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p,
                                               ctypes.c_void_p]
+    lib.mgatk_deletion_scan_device.argtypes = [ctypes.c_void_p, ctypes.POINTER(ParamsC), ctypes.POINTER(MgatkBatchC),
+                                               ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32,
+                                               ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                               ctypes.c_void_p]
     if lib.mgatk_abi_version() != ABI_VERSION:
         raise ExtensionMissingError(f"ABI mismatch: library {lib.mgatk_abi_version()}, binding {ABI_VERSION}")
     _lib = lib

@@ -15,6 +15,7 @@
 #include "variants.cuh"
 #include "clones.cuh"
 #include "markers.cuh"
+#include "deletions.cuh"
 
 using namespace mgatk;
 
@@ -138,6 +139,8 @@ struct mgatk_handle {
     DevBuf clone_x;
     // clone markers: the nonzero (x, label) pairs of every variant, the fallback's ping-pong pairs, the counters
     DevBuf marker_scratch;
+    // deletions: sorted deletions, start bitmap, list of relevant records, dedup table
+    DevBuf del_scratch;
 };
 
 namespace {
@@ -576,6 +579,7 @@ int mgatk_destroy(mgatk_handle *h) {
     if (h->var_table.p) cudaFree(h->var_table.p);
     if (h->clone_x.p) cudaFree(h->clone_x.p);
     if (h->marker_scratch.p) cudaFree(h->marker_scratch.p);
+    if (h->del_scratch.p) cudaFree(h->del_scratch.p);
     if (h->s_h2d) { cudaStreamDestroy(h->s_h2d); cudaStreamDestroy(h->s_d2h); }
     if (h->events_ready) for (int i = 0; i <= kMaxStages; i++) cudaEventDestroy(h->ev[i]);
     if (h->stream) cudaStreamDestroy(h->stream);
@@ -676,6 +680,7 @@ int mgatk_check_stats(const mgatk_stats *st) {
     if (st->error_bits & ERR_EXTENT) return MGATK_ERR_EXTENT;
     if (st->error_bits & ERR_OVERFLOW_CAP) return MGATK_ERR_OVERFLOW_CAP;
     if (st->error_bits & ERR_SATURATED) return MGATK_ERR_STREAM_SATURATED;
+    if (st->error_bits & ERR_DEL_RANGE) return MGATK_ERR_RANGE;
     return MGATK_OK;
 }
 
@@ -898,6 +903,74 @@ int mgatk_marker_ranks_device(mgatk_handle *h, const uint32_t *counts_dev, const
     k_marker_rank<<<grid, kMarkerThreads, smem, s>>>((u64 *)base, (int32_t *)(base + o_labs), nnz, gsize, npop, n_cells,
                                                      n_variants, n_groups, (u64 *)(base + o_tkeys),
                                                      (int32_t *)(base + o_tlabs), (u64 *)rank2_out, (u64 *)ties_out);
+    CU(cudaGetLastError());
+    return MGATK_OK;
+}
+
+int mgatk_deletion_scan_device(mgatk_handle *h, const mgatk_params *p, const mgatk_batch *b, int32_t min_clip,
+                               const int32_t *left_dev, const int32_t *right_dev, int32_t n_deletions,
+                               uint32_t *counts_out, uint64_t *clip_hist_out, uint64_t *clip_seq_out,
+                               uint64_t *error_bits_out, void *stream) {
+    if (!h) return MGATK_ERR_BAD_ARG;
+    h->err.clear();
+    if (!p || !b || !error_bits_out) return fail(h, MGATK_ERR_BAD_ARG, "null argument");
+    if (b->n_records < 0 || p->n_cells < 0 || p->mito_length <= 0 || b->blob_bytes < 0 || n_deletions < 0)
+        return fail(h, MGATK_ERR_BAD_ARG, "negative size");
+    if (p->dedup_mode < 0 || p->dedup_mode > 2) return fail(h, MGATK_ERR_BAD_ARG, "dedup_mode must be 0, 1 or 2");
+    if (min_clip < 1) return fail(h, MGATK_ERR_BAD_ARG, "min_clip must be >= 1");
+    if (p->max_read_extent < 1) return fail(h, MGATK_ERR_BAD_ARG, "max_read_extent must be >= 1");
+    if ((clip_hist_out == nullptr) != (clip_seq_out == nullptr))
+        return fail(h, MGATK_ERR_BAD_ARG, "clip_hist_out and clip_seq_out go together");
+    if (n_deletions > 0 && (!left_dev || !right_dev || (p->n_cells > 0 && !counts_out)))
+        return fail(h, MGATK_ERR_BAD_ARG, "null deletion array");
+    if (b->n_records > 0 && (!b->pos || !b->tlen || !b->flag || !b->mapq || !b->bc_idx || !b->l_seq || !b->n_cigar || !b->blob_off))
+        return fail(h, MGATK_ERR_BAD_ARG, "null batch array");
+    if (b->blob_bytes > 0 && !b->blob) return fail(h, MGATK_ERR_BAD_ARG, "null blob");
+    if (((uintptr_t)b->blob & 15) != 0) return fail(h, MGATK_ERR_BAD_ARG, "blob must be 16-byte aligned");
+    if (p->max_read_extent > (1 << 20)) return fail(h, MGATK_ERR_EXTENT, "max_read_extent above 2^20");
+    if (n_deletions > MGATK_DEL_MAX) return fail(h, MGATK_ERR_RANGE, "more than MGATK_DEL_MAX deletions");
+    if (p->mito_length >= (1 << 24)) return fail(h, MGATK_ERR_RANGE, "mito_length must be below 2^24");
+    if (b->n_records >= (int64_t)0x7fffff00) return fail(h, MGATK_ERR_RANGE, "at most 2^31-257 records per batch");
+    const bool discover = clip_hist_out != nullptr;
+    if (b->n_records == 0 || (n_deletions == 0 && !discover)) return MGATK_OK;
+    CU(cudaSetDevice(h->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    const int64_t n = b->n_records;
+    u64 bits = 32, table_max = 1024;
+    while (bits < (u64)p->mito_length) bits <<= 1;
+    while (table_max < 2ull * (u64)n) table_max <<= 1;
+    const size_t o_byl = 256, o_byr = o_byl + align_up(kDelMax * 8), o_dl = o_byr + align_up(kDelMax * 8);
+    const size_t o_dr = o_dl + align_up(kDelMax * 4), o_bitmap = o_dr + align_up(kDelMax * 4);
+    const size_t o_rel = o_bitmap + align_up(bits / 8), o_table = o_rel + align_up((size_t)n * 4);
+    int rc = ensure(h, h->del_scratch, o_table + (size_t)table_max * sizeof(DelEntry));
+    if (rc) return rc;
+    char *base = (char *)h->del_scratch.p;
+    DelArgs a;
+    a.b = *b; a.n_cells = p->n_cells; a.P = p->mito_length; a.extent = p->max_read_extent; a.min_mapq = p->min_mapq;
+    a.dedup_mode = p->dedup_mode; a.min_clip = min_clip; a.n_del = n_deletions; a.discover = discover ? 1 : 0;
+    a.bitmap_mask = (u32)(bits - 1);
+    a.left = left_dev; a.right = right_dev;
+    a.by_l = (int2 *)(base + o_byl); a.by_r = (int2 *)(base + o_byr); a.dl = (int32_t *)(base + o_dl); a.dr = (int32_t *)(base + o_dr);
+    a.n_rel = (u32 *)base; a.rel = (u32 *)(base + o_rel); a.bitmap = (u32 *)(base + o_bitmap);
+    a.table = (DelEntry *)(base + o_table); a.table_max = table_max;
+    a.counts = counts_out; a.clip_hist = (u64 *)clip_hist_out; a.clip_seq = (u64 *)clip_seq_out; a.error_bits = (u64 *)error_bits_out;
+    CU(cudaMemsetAsync(base, 0, 4, s));
+    CU(cudaMemsetAsync(a.bitmap, 0, bits / 8, s));
+    h->launches = 0;
+    if (n_deletions > 0) { k_del_prep<<<1, kDelPrepThreads, 0, s>>>(a); h->launches++; }
+    const int64_t want = (n + kDelThreads - 1) / kDelThreads;
+    const unsigned grid = (unsigned)(want < 8 * h->sm_count ? want : 8 * h->sm_count);
+    const unsigned wide = (unsigned)(8 * h->sm_count);            // passes over the relevant records: their count stays on the device
+    k_del_relevance<<<grid, kDelThreads, 0, s>>>(a);
+    h->launches++;
+    if (p->dedup_mode != MGATK_DEDUP_NONE) {
+        k_del_clear<<<wide, kDelThreads, 0, s>>>(a);
+        k_del_insert<<<wide, kDelThreads, 0, s>>>(a);
+        k_del_min<<<grid, kDelThreads, 0, s>>>(a);
+        h->launches += 3;
+    }
+    k_del_count<<<wide, kDelThreads, 0, s>>>(a);
+    h->launches++;
     CU(cudaGetLastError());
     return MGATK_OK;
 }

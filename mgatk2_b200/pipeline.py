@@ -39,11 +39,15 @@ class MtDNAPipeline:
                  output_format: str = "standard", barcode_metadata=None, sample_name: str = "mgatk2",
                  report_title: str | None = None, report_subtitle: str | None = None, working_directory: str | None = None,
                  device: int = 0, devices: list | None = None, max_batch_records: int | None = None,
-                 call_variants: bool = False, find_clones: bool = False, clone_markers: bool = False):
+                 call_variants: bool = False, find_clones: bool = False, clone_markers: bool = False,
+                 deletions: list | None = None, find_deletions: bool = False):
         """`call_variants=True` adds `output/variant_stats.tsv.gz` and `output/variant_cells.tsv.gz` (variants.py) after
         the reference's outputs, which stay as they are. `find_clones=True` implies it and adds `output/clones.tsv.gz` and
         `output/clone_variants.tsv.gz` (clones.py, the called variants, default parameters). `clone_markers=True` implies
-        `find_clones` and adds `output/clone_markers.tsv.gz` (markers.py: each clone against the other graph cells)."""
+        `find_clones` and adds `output/clone_markers.tsv.gz` (markers.py: each clone against the other graph cells).
+        `deletions` (1-based HGVS ranges (first, last)) and `find_deletions=True` add one more pass over the same records
+        (deletions.py): `output/deletions.tsv.gz` per cell and deletion, and with `find_deletions` the breakpoint pairs
+        found from soft clips in `output/deletion_candidates.tsv.gz`, which are counted too."""
         self.bam_path = Path(bam_path)
         self.barcodes = set(barcodes)
         self.barcode_list = list(barcodes)
@@ -58,6 +62,8 @@ class MtDNAPipeline:
         self.clone_markers = bool(clone_markers)
         self.find_clones = bool(find_clones) or self.clone_markers
         self.call_variants = bool(call_variants) or self.find_clones
+        self.deletions = None if deletions is None else [(int(f), int(t)) for f, t in deletions]
+        self.find_deletions = bool(find_deletions)
         if not self.bam_path.exists():
             raise InvalidInputError(f"BAM file not found: {bam_path}")
         from .bamio import BamFile, pick_mito_contig
@@ -109,6 +115,17 @@ class MtDNAPipeline:
                     from .markers import clone_markers, write_clone_markers
                     write_clone_markers(clone_markers(src, clones, counts=counts),
                                         self.output_dir / "output" / "clone_markers.tsv.gz")
+        if self.deletions is not None or self.find_deletions:
+            from .deletions import run_deletion_files
+            t_del = time.time()
+            one = getattr(reader, "batch", None)             # a one-batch input is still in memory; a stream is re-read
+            parts_of = (lambda: iter([one])) if one is not None else reader._parts
+            cands = run_deletion_files(parts_of, reads_by_barcode.result, self.config, self.barcode_list,
+                                       self.output_dir / "output", deletions=self.deletions, find=self.find_deletions,
+                                       device=self.device)
+            reader.timings["deletions_s"] = time.time() - t_del
+            logger.info("deletions: %d given, %s found", len(self.deletions or []),
+                        "-" if cands is None else len(cands))
         self.timings = dict(getattr(reader, "timings", {}), write_s=time.time() - t_write, total_s=time.time() - start)
         c = self.config
         write_run_summary({                                               # analysis/qc.py:68-93
@@ -131,9 +148,10 @@ class MtDNAPipeline:
 def run_pipeline(bam_path: str, output_dir: str, barcode_file: str | None = None, min_barcode_reads: int = 10,
                  barcode_tag: str = "CB", mito_chr: str = "chrM", output_format: str = "standard", device: int = 0,
                  devices: list | None = None, max_batch_records: int | None = None, call_variants: bool = False,
-                 find_clones: bool = False, clone_markers: bool = False, **config_kwargs) -> dict:
+                 find_clones: bool = False, clone_markers: bool = False, deletions: list | None = None,
+                 find_deletions: bool = False, **config_kwargs) -> dict:
     """core.pipeline.run_pipeline (pipeline.py:184-270): whitelist from file / singlecell.csv / the BAM itself, then
-    `MtDNAPipeline.run()` (`call_variants`, `find_clones`, `clone_markers`: as there). `config_kwargs` are `PipelineConfig` keywords (min_baseq, min_mapq, max_strand_bias,
+    `MtDNAPipeline.run()` (`call_variants`, `find_clones`, `clone_markers`, `deletions`, `find_deletions`: as there). `config_kwargs` are `PipelineConfig` keywords (min_baseq, min_mapq, max_strand_bias,
     skip_deduplication, use_fragment_length_dedup, min_reads_per_cell, ...)."""
     barcodes, metadata = load_barcodes(barcode_file, bam_path, barcode_tag=barcode_tag, mito_chr=mito_chr,
                                        min_barcode_reads=min_barcode_reads)
@@ -141,4 +159,5 @@ def run_pipeline(bam_path: str, output_dir: str, barcode_file: str | None = None
     return MtDNAPipeline(bam_path, barcodes, Path(output_dir), config, output_format=output_format,
                          barcode_metadata=metadata, device=device, devices=devices,
                          max_batch_records=max_batch_records, call_variants=call_variants,
-                         find_clones=find_clones, clone_markers=clone_markers).run()
+                         find_clones=find_clones, clone_markers=clone_markers, deletions=deletions,
+                         find_deletions=find_deletions).run()

@@ -152,6 +152,7 @@ class BAMReader:
                 first_seen = np.full(max(n_wl, 1), np.iinfo(np.int64).max, np.int64)
                 first_seen[cells] = first_idx
                 self.streamed = False
+                self.batch = batch              # the one batch, for a later pass over the same records (deletions.py)
             else:
                 counts = None
                 plane_bytes = 11 * 2 * ((int(self.config.mito_length) + 63) // 64 * 64)
@@ -161,6 +162,7 @@ class BAMReader:
                 res = dispatch.run_stream(itertools.chain([first, second], parts), self.config, n_wl, self.devices,
                                           records_per_barcode=counts, first_seen=first_seen)
                 self.streamed = True
+                self.batch = None
             self.timings["gpu_host_abi_s"] = time.perf_counter() - t0
             if res.stats["n_empty_seq"]:
                 raise ValueError("record without SEQ passed the filters")       # readers.py:157 raises here

@@ -191,3 +191,68 @@ def synth_batch(n_cells: int, n_records: int, profile: str = "atac50", seed: int
     return ReadBatch(pos=pos, tlen=tlen, flag=flag, mapq=mapq, bc_idx=bc,
                      l_seq=np.full(n, L, np.uint16), n_cigar=ncig.astype(np.uint16),
                      blob_off=off.astype(np.uint32), blob=blob)
+
+
+def synth_deletions(n_cells: int = 40, n_fragments: int = 6000, deletions=((8470, 13446), (6330, 13994), (1500, 2100)),
+                    read_len: int = 50, mito_length: int = MITO_LENGTH, seed: int = 20261022, gap_reads: bool = True,
+                    n_background: int = 4000, skew: float = 0.0, het_levels=(0.0, 0.1, 0.3, 0.6, 0.9)):
+    """Reads of cells that carry large deletions (1-based HGVS ranges) at chosen heteroplasmy, on a seeded reference.
+
+    Every fragment lies at a breakpoint of one deletion. With the cell's heteroplasmy of that deletion it comes from a
+    deleted molecule (ref[:l + 1] + ref[r:], l = first - 2, r = last) and crosses the junction: it is aligned on its
+    longer side with a soft clip of the other side, which is added as a 0x800 supplementary record (hard-clipped). Else
+    it is a wild-type read over the breakpoint; some of those end exactly at l without a clip. Per deletion there is one
+    read with a D gap over the deleted segment (`gap_reads`) and two duplicates whose first copy shadows a junction read:
+    one with mapq 0, one without a clip (not relevant). `n_background` plain reads cover the contig so that the reference
+    vote recovers the reference; `skew` > 0 draws cells from lognormal weights of that sigma. Returns (ReadBatch, the
+    reference as a string, heteroplasmy float [n_cells, D] of the draw)."""
+    rng = np.random.default_rng(seed)
+    P, L = int(mito_length), int(read_len)
+    ref = "".join(np.array(list("ACGT"))[rng.integers(0, 4, P)])
+    lr = [(int(f) - 2, int(t)) for f, t in deletions]
+    D = len(lr)
+    het = np.array(het_levels)[rng.integers(0, len(het_levels), size=(n_cells, max(D, 1)))][:, :D]
+    w = rng.lognormal(0.0, skew, n_cells) if skew > 0 else np.ones(n_cells)
+    cells = _sample_categorical(rng, w, n_fragments)
+    recs = []
+
+    def add(pos, cigar, seq, cell, flag=None, mapq=60, tlen=None):
+        rev = bool(rng.random() < 0.5)
+        recs.append({"pos": int(pos), "cigar": cigar, "seq": seq, "bc_idx": int(cell),
+                     "flag": (147 if rev else 99) if flag is None else flag,
+                     "mapq": mapq, "tlen": int((-1 if rev else 1) * rng.integers(60, 400)) if tlen is None else tlen})
+
+    for k in range(n_fragments):
+        if D == 0:
+            break
+        cell, d = int(cells[k]), int(rng.integers(0, D))
+        l, r = lr[d]
+        mq = 60 if rng.random() < 0.95 else 10
+        if rng.random() < het[cell, d]:                      # deleted molecule over the junction
+            a = int(rng.integers(1, L))                       # bases up to l; the other L - a from r on
+            b = L - a
+            seq = ref[l + 1 - a: l + 1] + ref[r: r + b]
+            if a >= b:
+                add(l + 1 - a, [(0, a), (4, b)], seq, cell, mapq=mq)
+                add(r, [(5, a), (0, b)], ref[r: r + b], cell, flag=2048 | 0x1)
+            else:
+                add(r, [(4, a), (0, b)], seq, cell, mapq=mq)
+                add(l + 1 - a, [(0, a), (5, b)], ref[l + 1 - a: l + 1], cell, flag=2048 | 0x1)
+        else:                                                 # wild type over l / l + 1 or r - 1 / r
+            at = l if rng.random() < 0.5 else r - 1
+            s = at - L + 1 if (at == l and rng.random() < 0.1) else int(rng.integers(at - L + 2, at + 1))
+            add(s, [(0, L)], ref[s: s + L], cell, mapq=mq)
+    for d, (l, r) in enumerate(lr):
+        cell = d % n_cells
+        if gap_reads:
+            add(l - 20, [(0, 21), (2, r - l - 1), (0, L - 21)], ref[l - 20: l + 1] + ref[r: r + L - 21], cell)
+        b = L // 2
+        clip_seq = ref[l + 1 - (L - b): l + 1] + ref[r: r + b]
+        for first in ({"mapq": 0, "cigar": [(4, L - b), (0, b)], "seq": clip_seq},
+                      {"mapq": 60, "cigar": [(0, L)], "seq": ref[r: r + L]}):
+            add(r, first["cigar"], first["seq"], cell, flag=99, mapq=first["mapq"], tlen=333)
+            add(r, [(4, L - b), (0, b)], clip_seq, cell, flag=99, tlen=333)        # shadowed by the one before
+    for s in rng.integers(0, P - L, n_background):
+        add(s, [(0, L)], ref[s: s + L], int(rng.integers(0, n_cells)), mapq=60)
+    order = sorted(range(len(recs)), key=lambda i: recs[i]["pos"])          # stable: duplicates keep their order
+    return ReadBatch.from_records([recs[i] for i in order]), ref, het
